@@ -12,11 +12,14 @@ The dense glue networks of the full model (SwinT, FPNs, fuser, SECOND, TransFusi
 of the hot path: the headline line times the hot path alone (`config.workload` says so) and the `c4`
 object of the same line times the whole camera+LiDAR frame with plain-torch glue nets around it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); every rank runs the same per-frame work on its
 own synthetic sample (weak scaling, no data-path collective -- the path shards by sample), the
 timed region is bracketed by barrier + cuda synchronize, time = max over ranks.
+
+--dump-outputs DIR writes the two BEV maps the last timed step returned (rank 0) as DIR/camera_bev.npy and
+DIR/lidar_bev.npy, float32; the inputs are seeded, so two builds can be compared output for output.
 
 --impl reference times the reference's CPU implementation of the path on the host cores
 (oracle/_ref extension for the sparse encoder, the restated QuickCumsum for bev_pool, the C port
@@ -287,6 +290,21 @@ class HotPath:
                              pairs=int((rb.nbr >= 0).sum())))
         del spconv
         return rows, int(feats.shape[0])
+
+
+DUMP_MAX_ELEMENTS = 7_500_000     # 30 MB of float32 per array: the two BEV maps stay under 64 MB in all
+
+
+def dump_outputs(directory, arrays):
+    """Write each array as <directory>/<name>.npy in float32.  An array of more than DUMP_MAX_ELEMENTS elements
+    is written as a fixed sample of its flattened elements (positions drawn from a generator seeded with its
+    size), the same positions in every run."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.size > DUMP_MAX_ELEMENTS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(a.size).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def time_ms(fn, n=20, warm=3):
@@ -643,6 +661,8 @@ def run_ours(args, rank, world, local_rank):
     e1.record()
     barrier()
     ms_per_step = max_over_ranks(e0.elapsed_time(e1)) / args.steps
+    # what the last timed replay returned, copied out after the timed region
+    outputs = {"camera_bev": gout[0].cpu().numpy(), "lidar_bev": gout[1].cpu().numpy()} if args.dump_outputs else None
     # --- stage times: each stage as its own graph, replayed back to back with events between them -------
     from bevfusion_b200.voxelize import voxelize_mean_fused
     L = hp.L
@@ -779,6 +799,9 @@ def run_ours(args, rank, world, local_rank):
 
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
+        del outputs
     # --- roofline of the dominant kernel + the north star's named kernel (bev_pool) --------
     x, pts = hp.device_inputs(seed=0)
     rows, n_vox = hp.encoder_work(pts)
@@ -1084,7 +1107,11 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip the reference-CUDA-kernels leg")
     ap.add_argument("--no-c4", action="store_true", help="skip the full camera+LiDAR frame with the glue nets")
     ap.add_argument("--no-c5", action="store_true", help="skip the high-resolution stress configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32, under 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

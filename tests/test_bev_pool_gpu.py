@@ -1,5 +1,5 @@
 """GPU parity tests for bev_pool: CUDA path (through the C ABI) vs the CPU oracle, the committed
-golden fixture, and the reference's own CUDA kernels (oracle/_ref) when present.
+golden fixture, and the stored outputs of the reference's own CUDA kernels (tests/refgold.py).
 Tolerances: ranks / perm / interval tables bit-exact; pooled features <= 1e-4 relative
 (BASELINE.json north_star); backward is a pure copy -> bit-exact."""
 import os
@@ -9,7 +9,7 @@ import pytest
 import torch
 
 import oracle
-from conftest import ref_module
+from refgold import Gold
 
 pytestmark = pytest.mark.gpu
 
@@ -149,27 +149,25 @@ def test_empty_and_single(cuda):
     assert float(out.sum()) == 80 and float(out[0, :, 0, 3, 2].sum()) == 80
 
 
-def test_vs_reference_cuda_kernel(cuda):
-    """the reference's own bev_pool CUDA kernels, compiled unmodified for sm_100."""
-    ref = ref_module("bev_pool_ext_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
-    from bevfusion_b200.bev_pool import bev_pool_ext
+def reference_case_kernel(cuda):
+    """inputs of test_vs_reference_cuda_kernel: sorted rows, tables, dims and an output gradient"""
     B, D, H, W, c = 1, 1, 64, 64, 80
     feats, coords = random_case(200000, c, B, D, H, W, seed=21, hot_cells=4)
     x, g, rs, starts, lengths, _ = sorted_inputs(feats, coords, B, D, H, W)
     args = [torch.from_numpy(a).to(cuda) for a in (x, g, lengths, starts)]
-    torch.cuda.synchronize()
-    ref_out = ref.bev_pool_forward(*args, B, D, H, W)      # legacy default stream
-    torch.cuda.synchronize()
-    out = bev_pool_ext.bev_pool_forward(*args, B, D, H, W)
-    assert rel_err(out.cpu().numpy(), ref_out.cpu().numpy()) <= 1e-4
-    og = torch.randn(B, D, H, W, c, device=cuda)
-    torch.cuda.synchronize()
-    ref_g = ref.bev_pool_backward(og, args[1], args[2], args[3], B, D, H, W)
-    torch.cuda.synchronize()
-    got_g = bev_pool_ext.bev_pool_backward(og, args[1], args[2], args[3], B, D, H, W)
-    assert torch.equal(ref_g, got_g)
+    og = torch.randn((B, D, H, W, c), generator=torch.Generator().manual_seed(22)).to(cuda)
+    return args, (B, D, H, W), og
+
+
+def test_vs_reference_cuda_kernel(cuda):
+    """the reference's own bev_pool CUDA kernels, compiled unmodified for sm_100."""
+    from bevfusion_b200.bev_pool import bev_pool_ext
+    gold = Gold("bev_pool_kernel")
+    args, dims, og = reference_case_kernel(cuda)
+    out = bev_pool_ext.bev_pool_forward(*args, *dims)
+    gold.close("forward", out, 1e-4)
+    got_g = bev_pool_ext.bev_pool_backward(og, args[1], args[2], args[3], *dims)
+    gold.exact("backward", got_g)
 
 
 def test_plan_full_size_c2_properties(cuda):
@@ -210,29 +208,25 @@ def test_plan_full_size_c2_properties(cuda):
     assert float(gflat[dropped].abs().sum()) == 0.0
 
 
-def test_plan_full_size_c2_vs_reference_cuda_kernel(cuda):
-    """BASELINE config C2 against the reference's OWN CUDA kernel (compiled unmodified into oracle/_ref): the reference
-    path materialises x[perm] (592 MB) and runs bev_pool_forward on the sorted rows with the interval tables; the plan
-    path pools the unsorted volume through perm.  Same cells, same rows per cell in the same order -> <= 1e-4 (in fact
-    equal up to the summation tree of the wide intervals)."""
-    ref = ref_module("bev_pool_ext_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
+def reference_case_c2(cuda):
+    """inputs of test_plan_full_size_c2_vs_reference_cuda_kernel: the C2 plan and a lifted volume"""
     from bevfusion_b200 import synthetic as S
     from bevfusion_b200.bev_pool import BEVPoolPlan
     geom, cfg = S.camera_geometry("C2", device=cuda)
     plan = BEVPoolPlan(geom, cfg["xbound"], cfg["ybound"], cfg["zbound"])
-    t = plan.tables
-    x = S.lifted_features("C2", device=cuda, seed=1)
+    return plan, S.lifted_features("C2", device=cuda, seed=1)
+
+
+def test_plan_full_size_c2_vs_reference_cuda_kernel(cuda):
+    """BASELINE config C2 against the reference's OWN CUDA kernel (compiled unmodified for sm_100): the reference
+    path materialises x[perm] (592 MB) and runs bev_pool_forward on the sorted rows with the interval tables; the plan
+    path pools the unsorted volume through perm.  Same cells, same rows per cell in the same order -> <= 1e-4 (in fact
+    equal up to the summation tree of the wide intervals)."""
+    gold = Gold("bev_pool_c2")
+    plan, x = reference_case_c2(cuda)
     out = plan.pool(x)                                               # [1, 1, 360, 360, 80]
-    xs = x.reshape(-1, 80)[t.perm[:t.n_kept].long()].contiguous()    # what bev_pool.py:94 hands the kernel
-    torch.cuda.synchronize()
-    ref_out = ref.bev_pool_forward(xs, t.geom.contiguous(), t.lengths.contiguous(), t.starts.contiguous(), 1, 1, 360, 360)
-    torch.cuda.synchronize()
-    assert tuple(ref_out.shape) == tuple(out.shape)
-    err = (out.double() - ref_out.double()).abs().max() / ref_out.double().abs().max()
-    assert float(err) <= 1e-4
-    assert bool(((out != 0) == (ref_out != 0)).all())
+    gold.close("forward", out, 1e-4)
+    gold.exact("nonzero", out != 0)
 
 
 @pytest.mark.parametrize("cfg_name", ["tiny", "C2"])

@@ -1,6 +1,6 @@
 """GPU parity tests for the sparse-conv path: rulebook (bit-exact as index sets / output order),
 implicit-GEMM conv and the SparseEncoder (<= 1e-4 relative, BASELINE.json north_star) against
-the CPU oracle, the committed reference fixtures and the reference's CUDA extension."""
+the CPU oracle, the committed reference fixtures and the stored outputs of the reference's CUDA extension."""
 import glob
 import os
 
@@ -9,7 +9,7 @@ import pytest
 import torch
 
 import oracle
-from conftest import ref_module
+from refgold import Gold
 
 pytestmark = pytest.mark.gpu
 
@@ -43,6 +43,18 @@ def random_sparse(n, shape, B, seed):
     z = flat % shape[2]; y = (flat // shape[2]) % shape[1]
     x = (flat // (shape[2] * shape[1])) % shape[0]; b = flat // (shape[2] * shape[1] * shape[0])
     return np.stack([b, x, y, z], 1).astype(np.int32)
+
+
+def pair_table(pairs, num):
+    """a rulebook as one canonical array: (offset, in, out) rows in ascending order"""
+    p, n = pairs.cpu().numpy(), num.cpu().numpy()
+    t = np.concatenate([np.stack([np.full(n[k], k), p[k, 0, :n[k]], p[k, 1, :n[k]]], 1)
+                        for k in range(p.shape[0])]).astype(np.int64)
+    return t[np.lexsort(t.T[::-1])]
+
+
+def out_grad(n, c, seed):
+    return torch.randn((n, c), generator=torch.Generator().manual_seed(seed))
 
 
 def pair_sets(pairs, num):
@@ -165,38 +177,29 @@ def test_dense_layouts(cuda):
     assert np.array_equal(zm, gold.transpose(0, 1, 4, 2, 3).reshape(B, c * shape[2], shape[0], shape[1]))
 
 
-def test_vs_reference_cuda_extension(cuda):
-    """rulebook + conv of the reference's own GPU path (sparse_conv_ext built for sm_100)."""
-    ref = ref_module("sparse_conv_ext_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
-    from bevfusion_b200.spconv import ops
+def reference_case_conv(cuda):
+    """inputs of test_vs_reference_cuda_extension: indices, features and one filter per geometry"""
     shape, B, n, cin, cout = [64, 60, 13], 2, 20000, 16, 32
-    idx = random_sparse(n, shape, B, seed=9)
+    idx = torch.from_numpy(random_sparse(n, shape, B, seed=9)).to(cuda)
     rng = np.random.default_rng(3)
     feat = torch.from_numpy(rng.standard_normal((n, cin)).astype(np.float32)).to(cuda)
-    ti = torch.from_numpy(idx).to(cuda)
-    prev = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = False       # the reference GEMM is torch::mm_out
-    try:
-        for name, (ks, st, pd, subm) in GEOMS.items():
-            W = torch.from_numpy((rng.standard_normal((*ks, cin, cout)) / 12).astype(np.float32)).to(cuda)
-            out_shape = shape if subm else oracle.conv_output_size(shape, ks, st, pd, [1, 1, 1])
-            r_out, r_pairs, r_num = ref.get_indice_pairs_3d(ti, B, out_shape, shape, ks, st, pd, [1, 1, 1],
-                                                            [0, 0, 0], int(subm), 0)
-            outids, pairs, num = ops.get_indice_pairs(ti, B, shape, ks, st, pd, 1, 0, subm)
-            assert torch.equal(outids, r_out), name                   # same outputs, same order
-            assert torch.equal(num, r_num), name
-            assert pair_sets(pairs.cpu().numpy(), num.cpu().numpy()) == pair_sets(
-                r_pairs.cpu().numpy(), r_num.cpu().numpy()), name
-            ref_feat = ref.indice_conv_fp32(feat, W, r_pairs, r_num, r_out.shape[0], 0, int(subm))
-            ours = ops.indice_conv(feat, W, r_pairs, r_num, r_out.shape[0], False, subm)   # drop-in call
-            assert rel_err(ours.cpu().numpy(), ref_feat.cpu().numpy()) <= 1e-4, name
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = prev
+    filters = {name: torch.from_numpy((rng.standard_normal((*GEOMS[name][0], cin, cout)) / 12).astype(np.float32)).to(cuda)
+               for name in GEOMS}
+    return idx, feat, filters, shape, B
 
 
-from oracle.reference_pipeline import reference_encoder_forward  # noqa: E402
+def test_vs_reference_cuda_extension(cuda):
+    """rulebook + conv of the reference's own GPU path (sparse_conv_ext built for sm_100)."""
+    from bevfusion_b200.spconv import ops
+    gold = Gold("spconv_conv")
+    idx, feat, filters, shape, B = reference_case_conv(cuda)
+    for name, (ks, st, pd, subm) in GEOMS.items():
+        outids, pairs, num = ops.get_indice_pairs(idx, B, shape, ks, st, pd, 1, 0, subm)
+        gold.exact(name + ".outids", outids)                          # same outputs, same order
+        gold.exact(name + ".num", num)
+        gold.exact(name + ".pairs", pair_table(pairs, num))
+        ours = ops.indice_conv(feat, filters[name], pairs, num, outids.shape[0], False, subm)   # drop-in call
+        gold.close(name + ".out", ours, 1e-4)
 
 
 def make_encoder(cuda, sparse_shape, seed=0):
@@ -213,9 +216,8 @@ def make_encoder(cuda, sparse_shape, seed=0):
     return m
 
 
-def test_encoder_fused_vs_modular_vs_reference(cuda):
-    """whole SparseEncoder on a small grid: fused-epilogue path == module-by-module path, and
-    both match the encoder executed with the reference CUDA extension."""
+def reference_case_encoder(cuda):
+    """inputs of test_encoder_fused_vs_modular_vs_reference: encoder, features, batch-sorted coordinates"""
     shape, B = [160, 160, 41], 2
     m = make_encoder(cuda, shape)
     rng = np.random.default_rng(0)
@@ -223,22 +225,20 @@ def test_encoder_fused_vs_modular_vs_reference(cuda):
     order = np.lexsort((idx[:, 3], idx[:, 2], idx[:, 1], idx[:, 0]))   # batch-sorted like the caller
     coors = torch.from_numpy(idx[order]).to(cuda)
     feats = torch.from_numpy(rng.standard_normal((coors.shape[0], 5)).astype(np.float32)).to(cuda)
+    return m, feats, coors, B
+
+
+def test_encoder_fused_vs_modular_vs_reference(cuda):
+    """whole SparseEncoder on a small grid: fused-epilogue path == module-by-module path, and
+    both match the encoder executed with the reference CUDA extension."""
+    m, feats, coors, B = reference_case_encoder(cuda)
     with torch.no_grad():
         modular = m(feats, coors, B, fused=False, precision=0)
         fused = m(feats, coors, B, fused=True, precision=0)
     assert tuple(fused.shape) == (B, 256, 20, 20)
     scale = float(modular.abs().max())
     assert float((fused - modular).abs().max()) <= 1e-4 * scale
-    ref = ref_module("sparse_conv_ext_ref")
-    if ref is not None:
-        prev = torch.backends.cuda.matmul.allow_tf32
-        torch.backends.cuda.matmul.allow_tf32 = False
-        try:
-            with torch.no_grad():
-                gold = reference_encoder_forward(ref, m, feats, coors, B)
-        finally:
-            torch.backends.cuda.matmul.allow_tf32 = prev
-        assert float((fused - gold).abs().max()) <= 1e-4 * float(gold.abs().max())
+    Gold("spconv_encoder").close("out", fused, 1e-4)
     if tc_available(cuda):
         with torch.no_grad():
             for prec in (1, 3):                                      # 3xTF32 and BF16x3 (default)
@@ -393,18 +393,27 @@ def test_native_plan_cuda_graph(cuda):
             assert bool(torch.equal(out, eager)), (seed, n)
 
 
-def test_lidar_branch_full_size(cuda):
-    """BASELINE config C3 end to end: voxelize -> mean -> SparseEncoder on the full
-    1440x1440x41 grid; layer sizes follow SURVEY.md App. D and the output is finite / sparse."""
+def reference_case_lidar(cuda):
+    """inputs of test_lidar_branch_full_size: encoder on the C3 grid, voxel means and coordinates"""
     from bevfusion_b200 import synthetic as S
     from bevfusion_b200.voxelize import Voxelization, voxelize_mean
     L = S.LIDAR_C3
     pts = torch.from_numpy(S.lidar_cloud(seed=0)).to(cuda)
     vox = Voxelization(L["voxel_size"], L["point_cloud_range"], L["max_num_points"], L["max_voxels"]).eval()
-    v, c, n = vox(pts)
-    assert v.shape[0] == 160000
-    feats, coords = voxelize_mean(v, c, n, 0)
-    m = make_encoder(cuda, L["sparse_shape"])
+    feats, coords = voxelize_mean(*vox(pts), 0)
+    return make_encoder(cuda, L["sparse_shape"]), feats, coords
+
+
+def active_cells(out):
+    """[B, C, H, W] -> packed bits of the BEV cells with any non-zero channel"""
+    return np.packbits((out != 0).any(1).cpu().numpy().reshape(-1))
+
+
+def test_lidar_branch_full_size(cuda):
+    """BASELINE config C3 end to end: voxelize -> mean -> SparseEncoder on the full
+    1440x1440x41 grid; layer sizes follow SURVEY.md App. D and the output is finite / sparse."""
+    m, feats, coords = reference_case_lidar(cuda)
+    assert feats.shape[0] == 160000
     with torch.no_grad():
         out = m(feats, coords, 1)
     assert tuple(out.shape) == (1, 256, 180, 180)
@@ -412,18 +421,10 @@ def test_lidar_branch_full_size(cuda):
     nz = (out.abs().sum(1) > 0).float().mean()
     assert 0.05 < float(nz) < 0.9
     # full-size parity: the same encoder run op by op through the reference's own CUDA extension
-    ref = ref_module("sparse_conv_ext_ref")
-    if ref is not None:
-        prev = torch.backends.cuda.matmul.allow_tf32
-        torch.backends.cuda.matmul.allow_tf32 = False
-        try:
-            with torch.no_grad():
-                gold = reference_encoder_forward(ref, m, feats, coords, 1)
-        finally:
-            torch.backends.cuda.matmul.allow_tf32 = prev
-        assert tuple(gold.shape) == tuple(out.shape)
-        assert bool(((gold != 0) == (out != 0)).float().mean() > 0.9999)      # same active BEV cells
-        assert float((out - gold).abs().max()) <= 1e-4 * float(gold.abs().max())
+    gold = Gold("spconv_lidar")
+    gold.close("out", out, 1e-4)
+    same = np.unpackbits(active_cells(out)) == np.unpackbits(gold["active_cells"])
+    assert same.mean() > 0.9999                                                # same active BEV cells
 
 
 @pytest.mark.parametrize("geom", list(GEOMS))
@@ -450,30 +451,29 @@ def test_backward_vs_oracle(cuda, geom, cin, cout):
         assert rel_err(dw.cpu().numpy(), gdw) <= 1e-4, "weight grad, precision %d" % prec
 
 
-def test_backward_vs_reference_cuda_extension(cuda):
-    ref = ref_module("sparse_conv_ext_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
-    from bevfusion_b200.spconv import ops
+def reference_case_backward(cuda):
+    """inputs of test_backward_vs_reference_cuda_extension: indices, features and one filter per geometry"""
     shape, B, n, cin, cout = [48, 40, 11], 2, 8000, 32, 64
     idx = torch.from_numpy(random_sparse(n, shape, B, seed=4)).to(cuda)
     rng = np.random.default_rng(5)
     feat = torch.from_numpy(rng.standard_normal((n, cin)).astype(np.float32)).to(cuda)
-    prev = torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        for name, (ks, st, pd, subm) in GEOMS.items():
-            W = torch.from_numpy((rng.standard_normal((*ks, cin, cout)) / 17).astype(np.float32)).to(cuda)
-            out_shape = shape if subm else oracle.conv_output_size(shape, ks, st, pd, [1, 1, 1])
-            r_out, r_pairs, r_num = ref.get_indice_pairs_3d(idx, B, out_shape, shape, ks, st, pd, [1, 1, 1],
-                                                            [0, 0, 0], int(subm), 0)
-            g = torch.randn(r_out.shape[0], cout, device=cuda)
-            r_din, r_dw = ref.indice_conv_backward_fp32(feat, W, g, r_pairs, r_num, 0, int(subm))
-            din, dw = ops.sparse_conv_ext.indice_conv_backward_fp32(feat, W, g, r_pairs, r_num, 0, int(subm))
-            assert rel_err(din.cpu().numpy(), r_din.cpu().numpy()) <= 1e-4, name
-            assert rel_err(dw.cpu().numpy(), r_dw.cpu().numpy().reshape(dw.shape)) <= 1e-4, name
-    finally:
-        torch.backends.cuda.matmul.allow_tf32 = prev
+    filters = {name: torch.from_numpy((rng.standard_normal((*GEOMS[name][0], cin, cout)) / 17).astype(np.float32)).to(cuda)
+               for name in GEOMS}
+    return idx, feat, filters, shape, B
+
+
+def test_backward_vs_reference_cuda_extension(cuda):
+    from bevfusion_b200.spconv import ops
+    gold = Gold("spconv_backward")
+    idx, feat, filters, shape, B = reference_case_backward(cuda)
+    for i, (name, (ks, st, pd, subm)) in enumerate(GEOMS.items()):
+        W = filters[name]
+        outids, pairs, num = ops.get_indice_pairs(idx, B, shape, ks, st, pd, 1, 0, subm)
+        gold.exact(name + ".outids", outids)                          # the rows the gradient is given for
+        g = out_grad(outids.shape[0], W.shape[-1], i).to(cuda)
+        din, dw = ops.sparse_conv_ext.indice_conv_backward_fp32(feat, W, g, pairs, num, 0, int(subm))
+        gold.close(name + ".din", din, 1e-4)
+        gold.close(name + ".dw", dw.reshape(W.shape), 1e-4)
 
 
 def test_module_autograd(cuda):

@@ -7,7 +7,7 @@ import pytest
 import torch
 
 import oracle
-from conftest import ref_module
+from refgold import Gold
 
 pytestmark = pytest.mark.gpu
 
@@ -96,23 +96,24 @@ def test_voxel_mean(cuda):
     assert float((feats - ref).abs().max()) <= 1e-5 * float(ref.abs().max())
 
 
-def test_vs_reference_cuda_kernel(cuda):
-    """the reference's deterministic GPU voxelizer (O(N^2) + serial kernel), compiled unmodified."""
-    ref = ref_module("voxel_layer_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
+def reference_case_voxelize():
+    """inputs of test_vs_reference_cuda_kernel: points, voxel size, range, max points, max voxels"""
     from bevfusion_b200 import synthetic as S
     L = S.LIDAR_C3
     pts = S.lidar_cloud(seed=1, sweeps=2)            # ~59 k points keeps the O(N^2) scan short
-    p = torch.from_numpy(pts).to(cuda)
-    mp, mv = 10, 20000
-    voxels = torch.zeros(mv, mp, 5, device=cuda)
-    coors = torch.zeros(mv, 3, dtype=torch.int32, device=cuda)
-    num = torch.zeros(mv, dtype=torch.int32, device=cuda)
-    m = ref.hard_voxelize(p, voxels, coors, num, L["voxel_size"], L["point_cloud_range"], mp, mv, 3, True)
-    assert m == mv
-    ours = run_ours(cuda, pts, L["voxel_size"], L["point_cloud_range"], mp, mv)
-    assert_same(ours, (voxels[:m].cpu().numpy(), coors[:m].cpu().numpy(), num[:m].cpu().numpy(), m))
+    return pts, L["voxel_size"], L["point_cloud_range"], 10, 20000
+
+
+def test_vs_reference_cuda_kernel(cuda):
+    """the reference's deterministic GPU voxelizer (O(N^2) + serial kernel), compiled unmodified."""
+    gold = Gold("hard_voxelize")
+    pts, vs, cr, mp, mv = reference_case_voxelize()
+    assert int(gold["voxel_num"]) == mv
+    v, c, n = run_ours(cuda, pts, vs, cr, mp, mv)
+    assert c.shape[0] == mv
+    gold.exact("coors", c)
+    gold.exact("num_points", n)
+    gold.exact("voxels", v)
 
 
 def test_stress_c5_voxel_grid(cuda):
@@ -236,36 +237,44 @@ def test_dynamic_scatter_edge_cases(cuda):
         voxel_layer.dynamic_point_to_voxel_forward(feats[:1], big, "median")
 
 
-@pytest.mark.parametrize("reduce_type", ["mean", "max", "sum"])
-def test_dynamic_scatter_vs_reference_cuda_extension(cuda, reduce_type):
-    """forward and backward against the reference's own kernels (scatter_points_cuda.cu) compiled
-    unmodified into oracle/_ref, on the dynamic voxelization of a LiDAR cloud."""
-    ref = ref_module("voxel_layer_ref")
-    if ref is None:
-        pytest.skip("oracle/_ref not built")
+def reference_case_scatter(cuda):
+    """inputs of test_dynamic_scatter_vs_reference_cuda_extension: LiDAR points and their voxel coordinates"""
     from bevfusion_b200 import synthetic as S
     from bevfusion_b200.voxelize import voxel_layer
     L = S.LIDAR_C3
     pts = torch.from_numpy(S.lidar_cloud(seed=3, sweeps=3)).to(cuda)
     coors = torch.zeros(pts.shape[0], 3, dtype=torch.int32, device=cuda)
     voxel_layer.dynamic_voxelize(pts, coors, L["voxel_size"], L["point_cloud_range"], 3)
+    return pts, coors
+
+
+def scatter_grad(red):
+    return torch.randn(red.shape, generator=torch.Generator().manual_seed(red.shape[0])).to(red.device)
+
+
+@pytest.mark.parametrize("reduce_type", ["mean", "max", "sum"])
+def test_dynamic_scatter_vs_reference_cuda_extension(cuda, reduce_type):
+    """forward and backward against the reference's own kernels (scatter_points_cuda.cu) compiled
+    unmodified for sm_100, on the dynamic voxelization of a LiDAR cloud."""
+    from bevfusion_b200.voxelize import voxel_layer
+    gold = Gold("dynamic_scatter_" + reduce_type)
+    pts, coors = reference_case_scatter(cuda)
     assert bool((coors < 0).any())                               # some points fall outside the range
-    r_red, r_oc, r_map, r_cnt = ref.dynamic_point_to_voxel_forward(pts, coors, reduce_type)
     red, oc, cmap, cnt = voxel_layer.dynamic_point_to_voxel_forward(pts, coors, reduce_type)
-    assert torch.equal(oc, r_oc.int()) and torch.equal(cmap, r_map.int()) and torch.equal(cnt, r_cnt.int())
+    gold.exact("out_coors", oc)
+    gold.exact("coors_map", cmap)
+    gold.exact("count", cnt)
     if reduce_type == "max":
-        assert torch.equal(red, r_red)
+        gold.exact("reduced", red)
     else:
-        assert float((red - r_red).abs().max()) <= 1e-5 * float(r_red.abs().max())
-    g = torch.randn_like(red)
-    r_grad = torch.zeros_like(pts)
-    ref.dynamic_point_to_voxel_backward(r_grad, g, pts, r_red, r_map, r_cnt, reduce_type)
+        gold.close("reduced", red, 1e-5)
+    g = scatter_grad(red)
     grad = torch.full_like(pts, float("nan"))
     voxel_layer.dynamic_point_to_voxel_backward(grad, g, pts, red, cmap, cnt, reduce_type)
     if reduce_type == "max":
-        assert torch.equal(grad, r_grad)
+        gold.exact("grad", grad)
     else:
-        assert float((grad - r_grad).abs().max()) <= 1e-6 * float(r_grad.abs().max())
+        gold.close("grad", grad, 1e-6)
 
 
 @pytest.mark.parametrize("average", [True, False])
