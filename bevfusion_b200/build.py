@@ -13,10 +13,6 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-gencode", "arch=compute_100a,code=sm_100a",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",
          "-Xptxas", "-warn-spills"]
-if os.environ.get("BEVB200_BUILD_NOHINT") == "1":
-    FLAGS.append("-DBEVB200_TC_NOHINT")
-if os.environ.get("BEVB200_BUILD_PROFILE") == "1":      # per-role cycle counters in the spconv kernel
-    FLAGS.append("-DBEVB200_TC_PROFILE")                # (tools/conv_prof.py); rebuild with --force
 
 
 def _stale(obj, src):

@@ -5,30 +5,25 @@
 // mmdet3d/ops/bev_pool/bev_pool.py:38-98, mmdet3d/models/vtransforms/base.py:141-176.
 //
 // B200 design (HBM-bound, ~0.64 GB per launch at the C2 workload):
-//   * the sorted row stream is cut into CHUNK_ROWS-row chunks; one warp owns one chunk, so
-//     work per warp is uniform no matter how skewed the interval lengths are (1 .. >1000)
-//   * an interval belongs to the chunk that holds its first row and is reduced by that warp
-//     alone, except intervals longer than 2*CHUNK_ROWS which are cut at chunk boundaries into
-//     pieces; pieces land in a small partial buffer and a second tiny kernel adds them in
-//     fixed order -> results are bit-reproducible run to run (no float atomics)
-//   * rows are read with 16-byte streaming loads (ld.global.nc.L1::no_allocate.v4), G rows x
-//     C/4 quads = T*32 float4 per warp step, two steps in flight (>= 2*T*512 B per warp)
-//   * the per-lane partial sums are folded through shared memory once per interval and the
-//     finished row is stored with one coalesced 16-byte-per-lane store
+//   * the sorted row stream is cut into equal ranges, one per warp, so work per warp is uniform no
+//     matter how skewed the interval lengths are (1 .. >1000); the forward streams each range
+//     through a shared-memory ring (see "forward" below), the backward walks CHUNK_ROWS-row chunks
+//   * an interval that crosses a range boundary leaves its pieces in a small partial buffer and a
+//     second tiny kernel adds them in fixed order -> results are bit-reproducible run to run (no
+//     float atomics)
 //   * `perm` variants read rows of the ORIGINAL feature tensor through the sorted->original
 //     map, which removes x[kept] / feats[indices] (2 x 0.6 GB of copies) from the frame
+// The first forward kernel (one warp per 128-row chunk, 16-byte register loads, per-interval folds
+// through shared memory) was removed after the TMA-staged kernel replaced it: DESIGN.md 4.1.
 #include <cub/device/device_radix_sort.cuh>
-
-#include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
 namespace bevb200 {
 
-constexpr int kChunkRows = 128;            // rows of the sorted stream owned by one warp
-constexpr int kLongRows = 2 * kChunkRows;  // intervals longer than this are cut into pieces
-constexpr int kPoolWarps = 8;              // warps per CTA
+constexpr int kChunkRows = 128;            // rows of the sorted stream owned by one backward warp (and the
+                                           // unit pool_partial_bytes sizes the forward's partial buffer in)
+constexpr int kPoolWarps = 8;              // warps per CTA of the backward kernel
 
 struct PoolDims {
   int b, d, h, w;
@@ -55,158 +50,7 @@ __device__ __forceinline__ int find_interval(const int32_t *__restrict__ starts,
 }
 
 // ---------------------------------------------------------------------------------------
-// forward
-// ---------------------------------------------------------------------------------------
-// Q = C/4 float4 per row, G rows per warp step, T = G*Q/32 float4 per lane per step.
-template <int Q, int G>
-struct PoolCfg {
-  static constexpr int T = G * Q / 32;
-  static_assert(G * Q % 32 == 0, "a warp step must be a whole number of float4 per lane");
-  static_assert(32 % G == 0, "G must divide the 32-row perm block");
-};
-
-template <int Q, int G>
-__device__ __forceinline__ void reduce_piece(const float4 *__restrict__ x,
-                                             const int32_t *__restrict__ perm, int s, int e,
-                                             float4 *__restrict__ dst, float4 *sm /*[G*Q]*/) {
-  constexpr int T = PoolCfg<Q, G>::T;
-  const int lane = lane_id();
-  int rig[T], qq[T];
-#pragma unroll
-  for (int t = 0; t < T; ++t) {
-    int f = lane + 32 * t;
-    rig[t] = f / Q;
-    qq[t] = f % Q;
-  }
-  float4 acc[T];
-#pragma unroll
-  for (int t = 0; t < T; ++t) acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
-
-  for (int r0 = s; r0 < e; r0 += 32) {
-    // source rows of this 32-row block, one per lane
-    int row = r0 + lane;
-    int src = row < e ? (perm ? __ldg(perm + row) : row) : 0;
-    const int nrows = min(32, e - r0);
-#pragma unroll 1
-    for (int g0 = 0; g0 < nrows; g0 += 2 * G) {
-      float4 va[T], vb[T];
-#pragma unroll
-      for (int t = 0; t < T; ++t) {
-        int ra = g0 + rig[t];
-        int sa = __shfl_sync(0xffffffffu, src, ra & 31);
-        va[t] = ra < nrows ? ldg_stream_f4(x + (long long)sa * Q + qq[t])
-                           : make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-      if (2 * G <= 32) {
-#pragma unroll
-        for (int t = 0; t < T; ++t) {
-          int rb = g0 + G + rig[t];
-          int sb = __shfl_sync(0xffffffffu, src, rb & 31);
-          vb[t] = rb < nrows ? ldg_stream_f4(x + (long long)sb * Q + qq[t])
-                             : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      }
-#pragma unroll
-      for (int t = 0; t < T; ++t) {
-        acc[t].x += va[t].x; acc[t].y += va[t].y; acc[t].z += va[t].z; acc[t].w += va[t].w;
-      }
-      if (2 * G <= 32) {
-#pragma unroll
-        for (int t = 0; t < T; ++t) {
-          acc[t].x += vb[t].x; acc[t].y += vb[t].y; acc[t].z += vb[t].z; acc[t].w += vb[t].w;
-        }
-      }
-    }
-  }
-  // fold the G row-slots of every quad (fixed order) and store the finished row
-  __syncwarp();
-#pragma unroll
-  for (int t = 0; t < T; ++t) sm[lane + 32 * t] = acc[t];
-  __syncwarp();
-  for (int q = lane; q < Q; q += 32) {
-    float4 r = sm[q];
-#pragma unroll
-    for (int g = 1; g < G; ++g) {
-      float4 v = sm[g * Q + q];
-      r.x += v.x; r.y += v.y; r.z += v.z; r.w += v.w;
-    }
-    dst[q] = r;
-  }
-  __syncwarp();
-}
-
-template <int Q, int G>
-__global__ void __launch_bounds__(kPoolWarps * 32)
-    bevpool_fwd_kernel(const float4 *__restrict__ x, const int32_t *__restrict__ perm,
-                       const int32_t *__restrict__ geom_feats,
-                       const int32_t *__restrict__ starts, const int32_t *__restrict__ lengths,
-                       int n, int n_intervals, PoolDims dm, float4 *__restrict__ out,
-                       float4 *__restrict__ partial) {
-  __shared__ float4 sm_all[kPoolWarps][G * Q];
-  float4 *sm = sm_all[threadIdx.x >> 5];
-  const int nchunks = (n + kChunkRows - 1) / kChunkRows;
-  const int warps_total = gridDim.x * kPoolWarps;
-  for (int j = blockIdx.x * kPoolWarps + (threadIdx.x >> 5); j < nchunks; j += warps_total) {
-    const int c0 = j * kChunkRows, c1 = min(n, c0 + kChunkRows);
-    int i = find_interval(starts, n_intervals, c0);
-    // (a) a long interval that began before this chunk and reaches into it
-    if (i >= 0) {
-      int s = __ldg(starts + i), L = __ldg(lengths + i);
-      if (s < c0 && L > kLongRows && s + L > c0)
-        reduce_piece<Q, G>(x, perm, c0, min(s + L, c1), partial + (2ll * j) * Q, sm);
-      if (s < c0) ++i;
-    } else {
-      i = 0;
-    }
-    // (b) intervals whose first row lies in this chunk
-    for (; i < n_intervals; ++i) {
-      int s = __ldg(starts + i);
-      if (s >= c1) break;
-      int L = __ldg(lengths + i);
-      if (L <= 0) continue;
-      int e = min(s + L, n);
-      if (L > kLongRows) {
-        reduce_piece<Q, G>(x, perm, s, min(e, c1), partial + (2ll * j + 1) * Q, sm);
-      } else {
-        long long cell = cell_of(geom_feats, s, dm);
-        if (cell >= 0) reduce_piece<Q, G>(x, perm, s, e, out + cell * Q, sm);
-      }
-    }
-  }
-}
-
-// adds the pieces of every long interval in chunk order (one warp per interval)
-template <int Q>
-__global__ void __launch_bounds__(256)
-    bevpool_fwd_fixup_kernel(const int32_t *__restrict__ geom_feats,
-                             const int32_t *__restrict__ starts,
-                             const int32_t *__restrict__ lengths, int n, int n_intervals,
-                             PoolDims dm, float4 *__restrict__ out,
-                             const float4 *__restrict__ partial) {
-  const int lane = lane_id();
-  const int warps_total = gridDim.x * (blockDim.x >> 5);
-  for (int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n_intervals;
-       i += warps_total) {
-    int L = __ldg(lengths + i);
-    if (L <= kLongRows) continue;
-    int s = __ldg(starts + i);
-    int e = min(s + L, n);
-    long long cell = cell_of(geom_feats, s, dm);
-    if (cell < 0 || e <= s) continue;
-    int jf = s / kChunkRows, jl = (e - 1) / kChunkRows;
-    for (int q = lane; q < Q; q += 32) {
-      float4 r = partial[(2ll * jf + 1) * Q + q];
-      for (int j = jf + 1; j <= jl; ++j) {
-        float4 v = partial[(2ll * j) * Q + q];
-        r.x += v.x; r.y += v.y; r.z += v.z; r.w += v.w;
-      }
-      out[cell * Q + q] = r;
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------
-// forward, v2: TMA-staged streaming reduction (the default for the tuned channel widths)
+// forward: TMA-staged streaming reduction (the tuned channel widths)
 // ---------------------------------------------------------------------------------------
 // Every warp owns a contiguous range of the sorted row stream and runs its own
 // cp.async.bulk -> shared memory ring (32 rows per stage, mbarrier complete_tx), so the bytes in
@@ -253,11 +97,11 @@ __global__ void pool_interval_cells_kernel(const int32_t *__restrict__ geom_feat
 struct LiftDims {
   int d_bins, hw;   // depth bins D and fH*fW: original index i -> pixel row (i / (D*hw)) * hw + i % hw
 };
-// MODE 3: rows gathered through perm with TMA tile::gather4 (4 rows per instruction; the tensor map
-// describes x as a 2-D [rows, C] fp32 tensor with a {C, 1} box; out-of-range row indices zero-fill).
+// (Gathering through perm with TMA tile::gather4, 4 rows per instruction, was measured no faster at C2 --
+// 166 us vs 162 us: row-granular gathers cap near 3.9 TB/s with either mechanism -- and removed.)
 template <int Q, int MODE>
 __global__ void __launch_bounds__(256)
-    bevpool_fwd_tma_kernel(const __grid_constant__ CUtensorMap xmap, const float4 *__restrict__ x,
+    bevpool_fwd_tma_kernel(const float4 *__restrict__ x,
                            const int32_t *__restrict__ perm, const float *__restrict__ depth, LiftDims lift,
                            const int32_t *__restrict__ starts, const int32_t *__restrict__ cells,
                            int n, int n_intervals, int rows_per_warp, int zfill, int total_cells,
@@ -313,22 +157,6 @@ __global__ void __launch_bounds__(256)
           asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + (uint32_t)f * 16u),
                        "l"(x + srow * Q + q) : "memory");
       }
-    } else if constexpr (MODE == 3) {
-      const uint32_t bar = bar0 + 8 * s;
-      const int prow = lane < nrows ? __ldg(perm + r0s + lane) : -1;   // -1: out of range -> zero fill
-      if (lane == 0)
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar),
-                     "r"((uint32_t)kStageRows * kRowBytes) : "memory");
-      const int i0 = __shfl_sync(0xffffffffu, prow, (4 * lane) & 31);
-      const int i1 = __shfl_sync(0xffffffffu, prow, (4 * lane + 1) & 31);
-      const int i2 = __shfl_sync(0xffffffffu, prow, (4 * lane + 2) & 31);
-      const int i3 = __shfl_sync(0xffffffffu, prow, (4 * lane + 3) & 31);
-      if (lane < kStageRows / 4)
-        asm volatile(
-            "cp.async.bulk.tensor.2d.shared::cluster.global.tile::gather4.mbarrier::complete_tx::bytes"
-            " [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-            ::"r"(dst + (uint32_t)lane * 4u * kRowBytes), "l"(&xmap), "r"(bar), "r"(0), "r"(i0), "r"(i1),
-              "r"(i2), "r"(i3) : "memory");
     } else {
       const uint32_t bar = bar0 + 8 * s;
       if (lane == 0) {
@@ -567,6 +395,14 @@ __global__ void bevpool_fwd_generic_kernel(const float *__restrict__ x,
 // ---------------------------------------------------------------------------------------
 // backward: x_grad[row, :] = out_grad[cell(interval(row)), :]
 // ---------------------------------------------------------------------------------------
+// Q = C/4 float4 per row, G rows per warp step, T = G*Q/32 float4 per lane per step.
+template <int Q, int G>
+struct PoolCfg {
+  static constexpr int T = G * Q / 32;
+  static_assert(G * Q % 32 == 0, "a warp step must be a whole number of float4 per lane");
+  static_assert(32 % G == 0, "G must divide the 32-row perm block");
+};
+
 template <int Q, int G>
 __global__ void __launch_bounds__(kPoolWarps * 32)
     bevpool_bwd_kernel(const float4 *__restrict__ out_grad, const int32_t *__restrict__ perm,
@@ -674,49 +510,6 @@ static size_t pool_partial_bytes(int n, int c) {
   return align_up(2 * nchunks * (size_t)c * sizeof(float)) + align_up((size_t)n * sizeof(int32_t));
 }
 
-template <int Q, int G>
-static int launch_fwd(const float *x, const int32_t *perm, const int32_t *geom,
-                      const int32_t *starts, const int32_t *lengths, int n, int n_intervals,
-                      PoolDims dm, float *out, float *partial, cudaStream_t st) {
-  int nchunks = (n + kChunkRows - 1) / kChunkRows;
-  int grid = min((nchunks + kPoolWarps - 1) / kPoolWarps, kNumSMs * 4);
-  BEVB200_LAUNCH((bevpool_fwd_kernel<Q, G>), grid, kPoolWarps * 32, 0, st, (const float4 *)x, perm,
-                 geom, starts, lengths, n, n_intervals, dm, (float4 *)out, (float4 *)partial);
-  int fgrid = min((n_intervals + 7) / 8, kNumSMs * 4);
-  BEVB200_LAUNCH((bevpool_fwd_fixup_kernel<Q>), fgrid, 256, 0, st, geom, starts, lengths, n,
-                 n_intervals, dm, (float4 *)out, (const float4 *)partial);
-  return BEVB200_OK;
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-// cuTensorMapEncodeTiled through the runtime's driver entry point table (no libcuda link)
-static EncodeTiledFn pool_encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void *p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess) fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
-// BEVB200_POOL_GATHER4=1 selects TMA tile::gather4 (4 rows per instruction) instead of the 16-byte
-// cp.async gather.  Measured at C2: 166 us vs 162 us -- row-granular gathers cap near 3.9 TB/s with
-// either mechanism -- so the simpler cp.async path is the default.
-static bool pool_gather4_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char *e = getenv("BEVB200_POOL_GATHER4");
-    on = (e && e[0] == '1') ? 1 : 0;
-    if (on && pool_encode_tiled() == nullptr) on = 0;
-  }
-  return on == 1;
-}
-
 template <int Q>
 static int launch_fwd_tma(const float *x, const int32_t *perm, const int32_t *geom,
                           const int32_t *starts, int n, int c, int n_intervals, PoolDims dm, float *out,
@@ -738,31 +531,15 @@ static int launch_fwd_tma(const float *x, const int32_t *perm, const int32_t *ge
   rpw = (rpw + kStageRows - 1) / kStageRows * kStageRows;
   const int n_ranges = (n + rpw - 1) / rpw;
   const int grid = (n_ranges + warps - 1) / warps;
-  // gathered rows: TMA gather4 needs a tensor map of x ([rows, C] fp32, box {C, 1}); the row count
-  // only bounds the zero-fill test, perm never points past the caller's tensor
-  CUtensorMap xmap;
-  memset(&xmap, 0, sizeof(xmap));
-  bool use_g4 = perm != nullptr && depth == nullptr && pool_gather4_enabled();
-  if (use_g4) {
-    cuuint64_t gdim[2] = {(cuuint64_t)c, (cuuint64_t)0x7fffffff};
-    cuuint64_t gstr[1] = {(cuuint64_t)c * 4};
-    cuuint32_t box[2] = {(cuuint32_t)c, 1};
-    cuuint32_t estr[2] = {1, 1};
-    if (pool_encode_tiled()(&xmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void *)x, gdim, gstr, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                            CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-      use_g4 = false;   // fall back to the cp.async gather
-  }
 #define BEVB200_POOL_TMA_LAUNCH(MODE)                                                             \
   do {                                                                                              \
     BEVB200_CUDA(cudaFuncSetAttribute(bevpool_fwd_tma_kernel<Q, MODE>,                              \
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));      \
-    BEVB200_LAUNCH((bevpool_fwd_tma_kernel<Q, MODE>), grid, warps * 32, smem, st, xmap,              \
+    BEVB200_LAUNCH((bevpool_fwd_tma_kernel<Q, MODE>), grid, warps * 32, smem, st,                    \
                    (const float4 *)x, perm, depth, lift, starts, cells, n, n_intervals, rpw, zfill,  \
                    dm.b * dm.d * dm.h * dm.w, (float4 *)out, (float4 *)partial);                     \
   } while (0)
   if (depth) BEVB200_POOL_TMA_LAUNCH(2);
-  else if (use_g4) BEVB200_POOL_TMA_LAUNCH(3);
   else if (perm) BEVB200_POOL_TMA_LAUNCH(1);
   else BEVB200_POOL_TMA_LAUNCH(0);
 #undef BEVB200_POOL_TMA_LAUNCH
@@ -795,10 +572,6 @@ static int launch_bwd(const float *og, const int32_t *perm, const int32_t *geom,
     default: FALLBACK; break;                    \
   }
 
-// 0 = TMA-staged streaming kernel (default), 1 = register-gather kernel (v1).  Selected by the
-// environment variable BEVB200_POOL_VARIANT at first use (kept for A/B measurements).
-static int g_pool_variant = -1;
-
 static int pool_forward(int b, int d, int h, int w, int n, int c, int n_intervals, const float *x,
                         const int32_t *perm, const int32_t *geom, const int32_t *starts,
                         const int32_t *lengths, float *out, void *ws, size_t ws_bytes,
@@ -808,10 +581,6 @@ static int pool_forward(int b, int d, int h, int w, int n, int c, int n_interval
   BEVB200_REQUIRE(out != nullptr, "null out");
   BEVB200_REQUIRE((long long)b * d * h * w * c < (1ll << 40), "output too large");
   BEVB200_REQUIRE((long long)b * d * h * w < (1ll << 31), "grid has too many cells");
-  if (g_pool_variant < 0) {
-    const char *e = getenv("BEVB200_POOL_VARIANT");
-    g_pool_variant = (e && e[0] == '1') ? 1 : 0;
-  }
   cudaStream_t st = (cudaStream_t)stream;
   size_t out_bytes = (size_t)b * d * h * w * c * sizeof(float);
   // plan tables (perm != null) with B*D == 1 are in ascending cell order: the pooling kernel
@@ -820,7 +589,7 @@ static int pool_forward(int b, int d, int h, int w, int n, int c, int n_interval
   switch (c) { case 16: case 32: case 64: case 80: case 96: case 128: case 160: case 256: tuned = true; }
   const bool aligned16 = ((uintptr_t)x % 16 == 0) && ((uintptr_t)out % 16 == 0);
   const int zfill = (perm != nullptr && b * d == 1 && n > 0 && n_intervals > 0 && tuned && aligned16 &&
-                     g_pool_variant == 0 && trust_tables) ? 1 : 0;
+                     trust_tables) ? 1 : 0;
   if (!zfill) BEVB200_CUDA(cudaMemsetAsync(out, 0, out_bytes, st));
   if (n == 0 || n_intervals == 0) return BEVB200_OK;
   BEVB200_REQUIRE(x && geom && starts && lengths, "null input");
@@ -834,10 +603,7 @@ static int pool_forward(int b, int d, int h, int w, int n, int c, int n_interval
                ws_bytes, pool_partial_bytes(n, c));                                            \
       return BEVB200_EWORKSPACE;                                                               \
     }                                                                                          \
-    if (g_pool_variant == 1)                                                                   \
-      rc = launch_fwd<Q, G>(x, perm, geom, starts, lengths, n, n_intervals, dm, out, (float *)ws, st); \
-    else                                                                                       \
-      rc = launch_fwd_tma<Q>(x, perm, geom, starts, n, c, n_intervals, dm, out, ws, zfill, st);  \
+    rc = launch_fwd_tma<Q>(x, perm, geom, starts, n, c, n_intervals, dm, out, ws, zfill, st);    \
   } while (0)
 #define CALL_FWD_GENERIC()                                                                     \
   do {                                                                                         \

@@ -457,6 +457,8 @@ int bevb200_encoder_create(int in_channels, const int32_t *sparse_shape_host, co
       cv.rulebook = (int)e->rulebooks.size();
       e->rulebooks.push_back(rb);
     }
+    // A residual is read from the source conv's SPLIT image -- hi + lo is the value to 2^-17 -- so only the last
+    // conv, whose rows dense() scatters, writes fp32 rows.
     cv.want_fp32 = i == n_convs - 1;
     cv.packed_off = poff; poff += align_up(spconv_v6_packed_bytes(cv.d.c_in, cv.d.c_out, cv.kvol));
     cv.scale_off = poff; poff += align_up((size_t)cv.d.c_out * 4);
@@ -465,11 +467,6 @@ int bevb200_encoder_create(int in_channels, const int32_t *sparse_shape_host, co
     e->convs.push_back(cv);
     c_prev = cv.d.c_out;
   }
-  // A residual is read from the source conv's SPLIT image -- hi + lo is the value to 2^-17 -- so only the last conv,
-  // whose rows dense() scatters, writes fp32 rows; BEVB200_ENCODER_F32_RESIDUAL=1 restores the fp32 residual copies.
-  static const bool f32_residual = [] { const char *v = getenv("BEVB200_ENCODER_F32_RESIDUAL"); return v && atoi(v) != 0; }();
-  for (EConv &cv : e->convs)
-    if (f32_residual && cv.d.residual_from >= 0) e->convs[cv.d.residual_from].want_fp32 = true;
   e->param_bytes = poff;
   *out = e;
   return BEVB200_OK;

@@ -1,4 +1,5 @@
-// Sparse convolution forward on the 5th-gen tensor cores (tcgen05 / TMEM), sm_100a only.
+// Sparse convolution forward on the 5th-gen tensor cores (tcgen05 / TMEM), sm_100a only: the TF32 modes
+// (generation 5) and the host dispatch of every precision.  BF16X3 runs generation 6 (spconv_v6.cu).
 //
 //   out[o, :] = epilogue( sum_k features[nbr[k, o], :] @ W[k] )          (spconv_ops.h:260-361)
 //
@@ -7,35 +8,33 @@
 // once, after the fused BN / residual / ReLU epilogue.  The GEMM K axis is the concatenation over
 // the kernel offsets of the Cin channels, cut into blocks of 32 floats (one 128-byte swizzle row).
 //
-// Default kernel (spconv_tc_kernel_v5, two CTAs per SM, 10 warps each; see the comment above it):
+// Kernel (spconv_tc_kernel_v5, two CTAs per SM, 10 warps each; see the comment above it):
 //   warps 0-3  GATHER: cp.async.cg 16-byte copies of the neighbour feature rows, 8 lanes per row =
 //              whole 128-byte lines, zero fill (ignore-src) for missing neighbours, into XOR-swizzled
 //              4 KB shared-memory staging slots; completion is signalled on an mbarrier by the
 //              copies themselves (cp.async.mbarrier.arrive.noinc).
 //   warps 4-7  CONVERT: lane = row; 8 conflict-free LDS.128 fetch the row's 32 floats, which are
-//              split into two parts (BF16x3: bf16 hi + bf16 lo; 3xTF32: tf32 hi + lo) in registers
-//              and written into TENSOR MEMORY with tcgen05.st (A ring of 2-4 stages).
-//   warp 8     one elected lane issues tcgen05.mma (kind::f16 / kind::tf32) with A from TMEM and B
-//              from shared memory (M128 x N=Cout x 32 B of K; per K step lo*hi + hi*lo + hi*hi, or
+//              split into two parts (3xTF32: tf32 hi + lo) in registers and written into TENSOR
+//              MEMORY with tcgen05.st (A ring of 2-4 stages).
+//   warp 8     one elected lane issues tcgen05.mma (kind::tf32) with A from TMEM and B from shared
+//              memory (M128 x N=Cout x 32 B of K; per K step lo*hi + hi*lo + hi*hi, or
 //              A_hi x [W_hi | W_lo] + A_lo x W_hi as two MMAs when Cout <= 64; fp32 accumulate),
 //              tcgen05.commit's the A / B ring slots back and finally the accumulator.
 //   warp 9     streams the weights: pre-packed in global memory as the exact K-major SWIZZLE_128B
 //              shared-memory image [hi | lo][Cout][128 B] and fetched with one cp.async.bulk
-//              (TMA 1-D) per stage into a ring (optionally multicast across a thread-block cluster).
+//              (TMA 1-D) per stage into a ring.
 //   epilogue   warps 0-7 read the accumulator with tcgen05.ld (32 lanes x 16 columns; warps w and
 //              w+4 share TMEM lane quarter w and split the columns), apply scale / shift (folded
 //              BatchNorm1d), residual and ReLU, and store the row.
-// Older generations stay selectable for A/B measurements (BEVB200_SPCONV_TC_VARIANT):
-//   4  spconv_tc_kernel_v4: same MMA / weight / epilogue roles, but 8 producer warps gather into
-//      registers (4 lanes per row), transpose with shuffles and split;
-//   (v2, both operands in shared memory, was removed: ncu showed it shared-memory bound -- every M128
-//   MMA re-reads its 4 KB A tile -- which is what moved A into TMEM; profiles/r1_conv_layers_v2.txt.)
+// Earlier generations were removed after their measurements (DESIGN.md 4.6):
+//   v2, both operands in shared memory (see below): profiles/r1_conv_layers_v2.txt.
+//   v4, 8 producer warps gathering into registers (4 lanes per row) + quad transposes: profiles/
+//   r1_conv_layers_v4.txt.  v5's own BF16x3 mode lost to generation 6: profiles/r1_conv_layers_v5_bf16x3.txt,
+//   r2_conv_v6_iterations.md.  Multicasting the weight stages across a thread-block cluster: no gain.
 //
-// Precision (all fp32 in, fp32 accumulate, fp32 out): BEVB200_PREC_BF16X3 (default; 5e-6 .. 8e-6 of
-// max|out| vs the float64 oracle), BEVB200_PREC_TF32X3 (1e-6 .. 1e-5), BEVB200_PREC_TF32 (single
-// pass, ~8e-4: below the 1e-4 parity bar, measurement only).
-#include <stdlib.h>
-
+// Precision (all fp32 in, fp32 accumulate, fp32 out): BEVB200_PREC_BF16X3 (default, generation 6;
+// 5e-6 .. 8e-6 of max|out| vs the float64 oracle), BEVB200_PREC_TF32X3 (1e-6 .. 1e-5), BEVB200_PREC_TF32
+// (single pass, ~8e-4: below the 1e-4 parity bar, measurement only).
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -48,15 +47,7 @@ constexpr int kKBlock = 32;                       // floats per K block = one 12
 
 constexpr int kMaxStages = 8;
 
-// Timing diagnostics (BEVB200_TC_DBG: 1 no staging reads, 2 no gather, 4 no MMA) produce WRONG outputs,
-// so they exist only in -DBEVB200_TC_PROFILE builds (BEVB200_BUILD_PROFILE=1 python bevfusion_b200/build.py).
-#ifdef BEVB200_TC_PROFILE
-#define TC_DBG(p, bit) ((p).dbg & (bit))
-#else
-#define TC_DBG(p, bit) 0
-#endif
-
-// ---- v4: A operand in TENSOR MEMORY (tcgen05.mma TS form) ------------------------------------
+// ---- A operand in TENSOR MEMORY (tcgen05.mma TS form) ----------------------------------------
 // Measured on v2 (removed): with both operands in shared memory the M128 x N x K8 tf32 MMA re-reads the
 // 4 KB A tile from smem on every instruction (3 per K step with the 3xTF32 split), which on top
 // of the producers' stores saturates the 128 B/clk shared-memory port -- the kernel was smem
@@ -66,9 +57,9 @@ constexpr int kMaxStages = 8;
 // fed by its own warp.  Layout of the 256 TMEM columns of a CTA (two CTAs per SM):
 //   [0, acc_cols)            fp32 accumulator, 128 lanes x Cout
 //   [acc_cols + 64*s ...)    A ring stage s: 32 columns hi | 32 columns lo   (K block of 32)
-constexpr int kV4Threads = 10 * 32;   // warps 0-7 producers/epilogue, 8 MMA issuer, 9 weight loader
+constexpr int kTcThreads = 10 * 32;   // warps 0-7 producers/epilogue, 8 MMA issuer, 9 weight loader
 
-struct TcParamsV4 {
+struct TcParams {
   const float *features;
   const float *wpacked;
   const int32_t *nbr;
@@ -79,12 +70,9 @@ struct TcParamsV4 {
   int nsa, nsb;       // TMEM A-ring stages, smem B-ring stages
   int acc_cols;       // accumulator columns (>= 32)
   int tmem_cols;      // allocation (power of two >= acc_cols + nsa * nsplit * 32)
-  long long *prof;    // optional: per-role cycle counters of CTA 0 (dev profiling)
   int nmerge;         // A_hi x [W_hi | W_lo] as ONE N = 2*c_out MMA (see the MMA issuer)
-  int nsg;            // v5: gather staging slots per row quarter (2..4, 4 KB each)
-  int nbr_bytes;      // v5: bytes of the neighbour table in shared memory (multiple of 128)
-  int csz;            // v5: thread-block cluster size (1, 2 or 4): weight stages are multicast
-  int dbg;            // timing diagnostics only (BEVB200_TC_DBG): 1 no staging reads, 2 no gather, 4 no MMA
+  int nsg;            // gather staging slots per row quarter (2..4, 4 KB each)
+  int nbr_bytes;      // bytes of the neighbour table in shared memory (multiple of 128)
 };
 
 __device__ __forceinline__ void tc_st16(uint32_t taddr, const uint32_t (&r)[16]) {
@@ -95,20 +83,6 @@ __device__ __forceinline__ void tc_st16(uint32_t taddr, const uint32_t (&r)[16])
         "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
       : "memory");
 }
-__device__ __forceinline__ void tc_st8(uint32_t taddr, const uint32_t (&r)[8]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-      : "memory");
-}
-__device__ __forceinline__ void tc_mma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc,
-                                               uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
 __device__ __forceinline__ void tc_mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc,
                                                uint32_t idesc, uint32_t accumulate) {
   asm volatile(
@@ -118,359 +92,14 @@ __device__ __forceinline__ void tc_mma_tf32_ts(uint32_t d_tmem, uint32_t a_tmem,
       ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
 
-// 4x4 transpose of float4 registers across the 4 lanes of a quad (lane & 3): after the call
-// a[c] on quad lane i holds what a[i] held on quad lane c.  Two butterfly rounds, 16 SHFL.
-__device__ __forceinline__ float4 shfl_xor_f4(const float4 &v, int m) {
-  float4 r;
-  r.x = __shfl_xor_sync(0xffffffffu, v.x, m);
-  r.y = __shfl_xor_sync(0xffffffffu, v.y, m);
-  r.z = __shfl_xor_sync(0xffffffffu, v.z, m);
-  r.w = __shfl_xor_sync(0xffffffffu, v.w, m);
-  return r;
-}
-__device__ __forceinline__ void quad_transpose(float4 (&a)[4], int lane) {
-  const bool b1 = (lane & 2) != 0, b0 = (lane & 1) != 0;
-  float4 x = b1 ? a[0] : a[2], y = b1 ? a[1] : a[3];
-  x = shfl_xor_f4(x, 2); y = shfl_xor_f4(y, 2);
-  if (b1) { a[0] = x; a[1] = y; } else { a[2] = x; a[3] = y; }
-  x = b0 ? a[0] : a[1]; y = b0 ? a[2] : a[3];
-  x = shfl_xor_f4(x, 1); y = shfl_xor_f4(y, 1);
-  if (b0) { a[0] = x; a[2] = y; } else { a[1] = x; a[3] = y; }
-}
-
-// Per-role cycle counters of CTA 0 (tools/conv_prof.py) are compiled in only with
-// -DBEVB200_TC_PROFILE (BEVB200_BUILD_PROFILE=1 python bevfusion_b200/build.py): the kernel is
-// instruction-issue bound, and the clock reads alone were 3 % of its instruction stream.
-#ifdef BEVB200_TC_PROFILE
-#define TC_PROF_CLOCK(var) const long long var = clock64()
-#define TC_PROF_ADD(cond, slot, val)              \
-  do {                                            \
-    if (p.prof && (cond)) p.prof[slot] += (val);  \
-  } while (0)
-#else
-#define TC_PROF_CLOCK(var) \
-  do {                     \
-  } while (0)
-#define TC_PROF_ADD(cond, slot, val) \
-  do {                               \
-  } while (0)
-#endif
-
-// ncu on the round-1 kernel (profiles/r1_ncu_full_final.md): issue slots 62 % busy, 2900 warp
-// instructions per K block per CTA of which ~750 were the gather / split / store work itself.  The
-// rest was loop bookkeeping, which this version removes: ring stage and phase are running
-// counters (no `it % nsa`, `it / nsa` with run-time divisors: ~20 integer divisions per K block),
-// a gather address is ONE IMAD.WIDE (base + row * row_bytes), the four neighbour indices of a quad
-// come from one LDS.128 instead of a load plus four shuffles, kernel parameters are read once, the
-// waits suspend on the mbarrier (try_wait with a time hint) instead of spinning, and the cycle
-// counters are compiled out.
-template <int NSPLIT>
-__global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v4(const TcParamsV4 p) {
-  TC_PROF_CLOCK(kernel_t0);
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t *smem = smem_raw + (smem_base - smem_u32(smem_raw));
-  // NSPLIT: 1 = single-pass TF32, 2 = 3xTF32 (hi/lo tf32 parts), 3 = BF16x3 (a = bf16 hi + bf16 lo;
-  // hi*hi + hi*lo + lo*hi with kind::f16: half the MMAs and half the operand bytes of 3xTF32 at
-  // 2^-17 per-product error).  In BF16 mode one 128-byte weight row holds 64 K values, i.e. one
-  // weight stage serves TWO 32-wide K blocks of A.
-  constexpr bool BF = NSPLIT == 3;
-  constexpr int NPART = BF ? 2 : NSPLIT;
-  const int c_out = p.c_out, nsa = p.nsa, nsb = p.nsb, n_iters = p.nkb;
-  const int b_part_bytes = c_out * 128;
-  const int b_stage_bytes = NPART * b_part_bytes;
-  __shared__ uint64_t bars[4 * kMaxStages + 1];
-  __shared__ uint32_t tmem_base_s;
-  const uint32_t a_full = smem_u32(&bars[0]), a_empty = smem_u32(&bars[kMaxStages]);
-  const uint32_t b_full = smem_u32(&bars[2 * kMaxStages]), b_empty = smem_u32(&bars[3 * kMaxStages]);
-  const uint32_t accbar = smem_u32(&bars[4 * kMaxStages]);
-  int32_t *nbr_s = reinterpret_cast<int32_t *>(smem + (size_t)nsb * b_stage_bytes);
-
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int row0 = blockIdx.x * kTileM;
-
-  if (tid == 0) {
-    for (int s = 0; s < nsa; ++s) {
-      mbar_init(a_full + 8 * s, 8);   // one arrival per producer warp
-      mbar_init(a_empty + 8 * s, 1);
-    }
-    for (int s = 0; s < nsb; ++s) {
-      mbar_init(b_full + 8 * s, 1);
-      mbar_init(b_empty + 8 * s, 1);
-    }
-    mbar_init(accbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 8) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(&tmem_base_s)), "r"((uint32_t)p.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_base_s;
-  const uint32_t a_ring = tmem_base + (uint32_t)p.acc_cols;            // column offset of A stage 0
-  constexpr uint32_t kAStageCols = BF ? 32u : (uint32_t)NSPLIT * 32u;   // BF16: 16 cols hi | 16 cols lo
-
-  if (warp < 8) {
-    // =============================== producers ===========================================
-    // TMEM lane quarter q = warp & 3 is the only one this warp may touch: row = 32 q + lane
-    const int q = warp & 3, half = warp >> 2;
-    {
-      // neighbour table of the tile: all (<= 14) loads of a thread are issued before any is used
-      constexpr int kPer = (27 * kTileM + kTcProducerThreads - 1) / kTcProducerThreads;
-      const int n_tab = p.kvol * kTileM, n_out = p.n_out, n_in = p.n_in;
-      int tv[kPer];
-#pragma unroll
-      for (int u = 0; u < kPer; ++u) {
-        const int i = tid + u * kTcProducerThreads;
-        const int k = i >> 7, rr = i & 127, o = row0 + rr;
-        tv[u] = (i < n_tab && o < n_out) ? __ldg(p.nbr + (long long)k * n_out + o) : -1;
-      }
-#pragma unroll
-      for (int u = 0; u < kPer; ++u) {
-        const int i = tid + u * kTcProducerThreads;
-        if (i < n_tab) nbr_s[i] = tv[u] >= n_in ? -1 : tv[u];
-      }
-    }
-    asm volatile("bar.sync 1, %0;" ::"n"(kTcProducerThreads) : "memory");
-
-    // Coalesced gather: load instruction t of a warp covers rows {4j + t : j = 0..7} of its
-    // quarter, 4 lanes x 16 B per row (64 contiguous bytes), so a warp-level LDG.128 touches 8
-    // cache lines instead of 32 (measured: the one-row-per-lane mapping was L1 wavefront bound).
-    // The quad transpose at consume time hands every lane the 64 bytes of ITS row.
-    const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-    const uint32_t row_bytes = (uint32_t)p.c_in * 4u;
-    const char *fbase = reinterpret_cast<const char *>(p.features) + 16 * (lane & 3);
-    const int32_t *nb_quad = nbr_s + q * 32 + (lane & ~3);   // the 4 rows of this lane's quad: one int4
-    const int cin_shift = p.cin_shift, cin_mask = p.c_in - 1, kvol = p.kvol;
-    auto issue = [&](int it, float4 (&v)[4]) {
-      const int kk = it * kKBlock + half * 16;
-      const int k = kk >> cin_shift;
-      const char *base = fbase + ((kk & cin_mask) << 2);
-      int4 s4 = make_int4(-1, -1, -1, -1);
-      if (k < kvol) s4 = *reinterpret_cast<const int4 *>(nb_quad + k * kTileM);
-      const int src[4] = {s4.x, s4.y, s4.z, s4.w};
-#pragma unroll
-      for (int t = 0; t < 4; ++t)
-        v[t] = src[t] >= 0 ? __ldg(reinterpret_cast<const float4 *>(
-                                 base + (unsigned long long)(uint32_t)src[t] * row_bytes))
-                           : make_float4(0.f, 0.f, 0.f, 0.f);
-    };
-    constexpr int PD = 3;   // K blocks prefetched in registers (4 spills under the 2-CTA/SM register cap)
-    float4 v[PD][4];
-#pragma unroll
-    for (int j = 0; j < PD; ++j)
-      if (j < n_iters) issue(j, v[j]);
-    int s = 0;              // A ring stage and its phase, advanced once per K block
-    uint32_t ph = 0;
-    const uint32_t col0 = a_ring + (uint32_t)(half * (BF ? 8 : 16));
-    for (int it0 = 0; it0 < n_iters; it0 += PD) {
-#pragma unroll
-      for (int jj = 0; jj < PD; ++jj) {
-        const int it = it0 + jj;
-        if (it < n_iters) {
-          TC_PROF_CLOCK(t0);
-          quad_transpose(v[jj], lane);
-          if (lane == 0) mbar_wait(a_empty + 8 * s, ph ^ 1u);   // one waiter per warp
-          __syncwarp();
-          tc_fence_after();
-          TC_PROF_CLOCK(t1);
-          const uint32_t col = lane_base + col0 + (uint32_t)s * kAStageCols;
-          if constexpr (BF) {
-            // 16 K values of this row -> 8 packed bf16 words hi + 8 words lo (k even in the low half)
-            uint32_t hi[8], lo[8];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float f[4] = {v[jj][j].x, v[jj][j].y, v[jj][j].z, v[jj][j].w};
-#pragma unroll
-              for (int e = 0; e < 4; e += 2) {
-                const uint32_t h = cvt_bf16x2(f[e + 1], f[e]);
-                const float h0 = __uint_as_float(h << 16), h1 = __uint_as_float(h & 0xffff0000u);
-                hi[2 * j + e / 2] = h;
-                lo[2 * j + e / 2] = cvt_bf16x2(f[e + 1] - h1, f[e] - h0);
-              }
-            }
-            tc_st8(col, hi);
-            tc_st8(col + 16u, lo);
-          } else {
-            uint32_t hi[16], lo[16];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float f[4] = {v[jj][j].x, v[jj][j].y, v[jj][j].z, v[jj][j].w};
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                hi[4 * j + e] = __float_as_uint(f[e]) & 0xffffe000u;
-                lo[4 * j + e] = __float_as_uint(f[e] - __uint_as_float(hi[4 * j + e]));
-              }
-            }
-            tc_st16(col, hi);
-            if (NSPLIT == 2) tc_st16(col + 32u, lo);
-          }
-          asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(a_full + 8 * s);            // 8 arrivals per K block, not 256
-          if (++s == nsa) { s = 0; ph ^= 1u; }
-          TC_PROF_CLOCK(t2);
-          if (it + PD < n_iters) issue(it + PD, v[jj]);
-          TC_PROF_ADD(blockIdx.x == 0 && tid == 0, 0, t1 - t0);             // transpose + wait for a free stage
-          TC_PROF_ADD(blockIdx.x == 0 && tid == 0, 1, t2 - t1);             // split + tcgen05.st + arrive
-          TC_PROF_ADD(blockIdx.x == 0 && tid == 0, 2, clock64() - t2);      // issue of the next gather loads
-        }
-      }
-    }
-    // =============================== epilogue ============================================
-    TC_PROF_CLOCK(e0);
-    mbar_wait(accbar, 0);
-    tc_fence_after();
-    TC_PROF_ADD(blockIdx.x == 0 && tid == 0, 3, clock64() - e0);   // drain: last MMAs
-    const int orow = row0 + q * 32 + lane;
-    const int ncol_half = c_out / 2;
-    const int col_begin = half * ncol_half;
-    const bool row_ok = orow < p.n_out;
-    const float *scale = p.scale, *shift = p.shift;
-    const int relu = p.relu;
-    for (int c0 = col_begin; c0 < col_begin + ncol_half; c0 += 16) {
-      float acc[16];
-      tc_ld16(tmem_base + lane_base + (uint32_t)c0, acc);
-      if (p.nmerge) {   // columns [c_out, 2 c_out) hold the hi x lo partial sums
-        float more[16];
-        tc_ld16(tmem_base + lane_base + (uint32_t)(c_out + c0), more);
-#pragma unroll
-        for (int e = 0; e < 16; ++e) acc[e] += more[e];
-      }
-      if (row_ok) {
-        float *dst = p.out + (long long)orow * c_out + c0;
-        const float *res = p.residual ? p.residual + (long long)orow * c_out + c0 : nullptr;
-        const int ncols = min(16, col_begin + ncol_half - c0);
-#pragma unroll
-        for (int j = 0; j < 16; j += 4) {
-          if (j < ncols) {
-            float y[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              float t = acc[j + e];
-              if (scale) t *= __ldg(scale + c0 + j + e);
-              if (shift) t += __ldg(shift + c0 + j + e);
-              y[e] = t;
-            }
-            if (res) {
-              const float4 rv = __ldg(reinterpret_cast<const float4 *>(res + j));
-              y[0] += rv.x; y[1] += rv.y; y[2] += rv.z; y[3] += rv.w;
-            }
-            if (relu) {
-#pragma unroll
-              for (int e = 0; e < 4; ++e) y[e] = fmaxf(y[e], 0.f);
-            }
-            *reinterpret_cast<float4 *>(dst + j) = make_float4(y[0], y[1], y[2], y[3]);
-          }
-        }
-      }
-    }
-  } else if (warp == 8) {
-    // =============================== MMA issuer ==========================================
-    const uint32_t idesc = BF ? umma_idesc_bf16(kTileM, c_out) : umma_idesc_tf32(kTileM, c_out);
-    const uint32_t idesc2 = BF ? umma_idesc_bf16(kTileM, 2 * c_out)   // merged [W_hi | W_lo] operand
-                               : umma_idesc_tf32(kTileM, 2 * c_out);
-    const int nmerge = p.nmerge;
-    int sa = 0, sb = 0;
-    uint32_t pa = 0, pb = 0;
-    for (int it = 0; it < n_iters; ++it) {
-      TC_PROF_CLOCK(m0);
-      mbar_wait(a_full + 8 * sa, pa);
-      TC_PROF_CLOCK(m1);
-      mbar_wait(b_full + 8 * sb, pb);   // BF16: already complete for the second K block of a stage
-      tc_fence_after();
-      TC_PROF_CLOCK(m2);
-      TC_PROF_ADD(blockIdx.x == 0 && lane == 0, 4, m1 - m0);
-      TC_PROF_ADD(blockIdx.x == 0 && lane == 0, 5, m2 - m1);
-      const bool last = it == n_iters - 1;
-      const bool b_done = !BF || (it & 1) || last;   // the weight stage is free after its last K block
-      if (elect_one_sync()) {
-        const uint32_t a_hi = a_ring + (uint32_t)sa * kAStageCols;   // lane 0, column offset
-        const uint32_t a_lo = a_hi + (BF ? 16u : 32u);
-        const uint32_t bstage = smem_base + (uint32_t)sb * (uint32_t)b_stage_bytes;
-        const uint64_t b_hi = umma_desc_sw128(bstage);
-        const uint64_t b_lo = umma_desc_sw128(bstage + b_part_bytes);
-        constexpr int KSTEPS = BF ? 2 : 4;           // 16 bf16 / 8 tf32 per MMA = 32 B of K either way
-#pragma unroll
-        for (int ks = 0; ks < KSTEPS; ++ks) {
-          // +32 B along K inside the 128-byte swizzled weight row (BF16: odd K blocks use its 2nd half)
-          const uint64_t badv = (uint64_t)(ks * 2 + (BF ? (it & 1) * 4 : 0));
-          const uint32_t aadv = (uint32_t)(ks * 8);   // 8 TMEM columns per K step (8 tf32 / 16 bf16)
-          const uint32_t d = tmem_base;
-          const uint32_t first = (it == 0 && ks == 0) ? 0u : 1u;
-          if (nmerge) {
-            // The hi and lo weight images are adjacent in the stage (same swizzle atoms), so one
-            // descriptor with N = 2*c_out multiplies A_hi by both: columns [0, c_out) collect
-            // hi*hi (+ lo*hi below), columns [c_out, 2 c_out) collect hi*lo.  2 MMAs, not 3; the
-            // epilogue adds the two column groups.
-            if constexpr (BF) {
-              tc_mma_bf16_ts(d, a_hi + aadv, b_hi + badv, idesc2, first);
-              tc_mma_bf16_ts(d, a_lo + aadv, b_hi + badv, idesc, 1u);
-            } else {
-              tc_mma_tf32_ts(d, a_hi + aadv, b_hi + badv, idesc2, first);
-              tc_mma_tf32_ts(d, a_lo + aadv, b_hi + badv, idesc, 1u);
-            }
-          } else if constexpr (BF) {
-            tc_mma_bf16_ts(d, a_lo + aadv, b_hi + badv, idesc, first);
-            tc_mma_bf16_ts(d, a_hi + aadv, b_lo + badv, idesc, 1u);
-            tc_mma_bf16_ts(d, a_hi + aadv, b_hi + badv, idesc, 1u);
-          } else if (NSPLIT == 2) {
-            tc_mma_tf32_ts(d, a_lo + aadv, b_hi + badv, idesc, first);
-            tc_mma_tf32_ts(d, a_hi + aadv, b_lo + badv, idesc, 1u);
-            tc_mma_tf32_ts(d, a_hi + aadv, b_hi + badv, idesc, 1u);
-          } else {
-            tc_mma_tf32_ts(d, a_hi + aadv, b_hi + badv, idesc, first);
-          }
-        }
-        tc_commit(a_empty + 8 * sa);
-        if (b_done) tc_commit(b_empty + 8 * sb);
-        if (last) tc_commit(accbar);
-        TC_PROF_ADD(blockIdx.x == 0, 6, clock64() - m2);   // MMA issue + commits
-      }
-      __syncwarp();
-      if (++sa == nsa) { sa = 0; pa ^= 1u; }
-      if (b_done && ++sb == nsb) { sb = 0; pb ^= 1u; }
-    }
-  } else {
-    // =============================== weight loader =======================================
-    if (lane == 0) {
-      const int n_bstages = BF ? (n_iters + 1) / 2 : n_iters;
-      const char *src = reinterpret_cast<const char *>(p.wpacked);
-      int sb = 0;
-      uint32_t pb = 1;   // an untouched stage counts as released
-      for (int it = 0; it < n_bstages; ++it) {
-        mbar_wait(b_empty + 8 * sb, pb);
-        mbar_arrive_expect_tx(b_full + 8 * sb, (uint32_t)b_stage_bytes);
-        bulk_copy_g2s(smem_base + (uint32_t)sb * (uint32_t)b_stage_bytes, src, (uint32_t)b_stage_bytes,
-                      b_full + 8 * sb);
-        src += b_stage_bytes;
-        if (++sb == nsb) { sb = 0; pb ^= 1u; }
-      }
-    }
-    __syncwarp();
-  }
-  tc_fence_before();
-  __syncthreads();
-  TC_PROF_ADD(blockIdx.x == 0 && tid == 0, 7, clock64() - kernel_t0);   // whole CTA
-  if (warp == 8) {
-    __syncwarp();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
-                 "r"((uint32_t)p.tmem_cols) : "memory");
-  }
-}
-
 // ---------------------------------------------------------------------------------------
 // v5: the gather goes through shared memory with cp.async, in WHOLE 128-byte lines.
 //
-// What bounded v4 after its instruction stream was trimmed: (1) a warp-level LDG is processed by
-// the L1 one 128-byte line at a time, ~2 clk per line whatever part of the line is used; v4's
-// 4-lanes-per-row loads touch 8 lines per instruction for 64 B each, 256 line-visits per K block per
-// CTA, ~530 clk with two CTAs sharing the SM's L1; (2) the 4x4 register transposes (16 SHFL + as
-// many selects per 16 floats) that turn "4 lanes per row" into "lane = row" for tcgen05.st.
+// What bounded v4 (register gather, since removed) after its instruction stream was trimmed: (1) a
+// warp-level LDG is processed by the L1 one 128-byte line at a time, ~2 clk per line whatever part of the
+// line is used; v4's 4-lanes-per-row loads touch 8 lines per instruction for 64 B each, 256 line-visits
+// per K block per CTA, ~530 clk with two CTAs sharing the SM's L1; (2) the 4x4 register transposes
+// (16 SHFL + as many selects per 16 floats) that turn "4 lanes per row" into "lane = row" for tcgen05.st.
 // v5 splits the producers into four GATHER warps and four CONVERT warps (one of each per TMEM lane
 // quarter):
 //   gather   lane (m, c) = (lane >> 3, lane & 7) copies the 16-byte chunk c of rows 8m+t, t = 0..7,
@@ -484,7 +113,6 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v4(const TcPar
 //            written to the TMEM A stage with tcgen05.st; arrive on a_full.
 // No data registers are held across the global-load latency (the slots are the prefetch buffer),
 // there is no shuffle, and each role's loop is ~55 / ~135 instructions per K block.
-// MMA issuer, weight loader and epilogue are v4's.
 // ---------------------------------------------------------------------------------------
 constexpr int kStageSlotBytes = 32 * 128;   // one quarter's rows of one K block
 constexpr int kMaxGatherSlots = 4;
@@ -495,16 +123,15 @@ __device__ __forceinline__ float4 lds128(uint32_t addr) {
   return v;
 }
 
+// NSPLIT: 1 = single-pass TF32, 2 = 3xTF32 (hi/lo tf32 parts)
 template <int NSPLIT>
-__global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcParamsV4 p) {
+__global__ void __launch_bounds__(kTcThreads, 2) spconv_tc_kernel_v5(const TcParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t *smem = smem_raw + (smem_base - smem_u32(smem_raw));
-  constexpr bool BF = NSPLIT == 3;
-  constexpr int NPART = BF ? 2 : NSPLIT;
-  const int c_out = p.c_out, nsa = p.nsa, nsb = p.nsb, nsg = p.nsg, n_iters = p.nkb, csz = p.csz;
+  const int c_out = p.c_out, nsa = p.nsa, nsb = p.nsb, nsg = p.nsg, n_iters = p.nkb;
   const int b_part_bytes = c_out * 128;
-  const int b_stage_bytes = NPART * b_part_bytes;
+  const int b_stage_bytes = NSPLIT * b_part_bytes;
   __shared__ uint64_t bars[4 * kMaxStages + 1 + 8 * kMaxGatherSlots];
   __shared__ uint32_t tmem_base_s;
   const uint32_t a_full = smem_u32(&bars[0]), a_empty = smem_u32(&bars[kMaxStages]);
@@ -526,7 +153,7 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
     }
     for (int s = 0; s < nsb; ++s) {
       mbar_init(b_full + 8 * s, 1);
-      mbar_init(b_empty + 8 * s, csz);   // released by the MMA warp of every CTA of the cluster
+      mbar_init(b_empty + 8 * s, 1);
     }
     for (int s = 0; s < 4 * kMaxGatherSlots; ++s) {
       mbar_init(g_full + 8 * s, 32);   // every lane of the gather warp: cp.async arrive (noinc)
@@ -542,12 +169,10 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
   }
   tc_fence_before();
   __syncthreads();
-  if (csz > 1) cluster_sync_all();        // peers' barriers are initialised before any multicast
   tc_fence_after();
-  const uint16_t cmask = (uint16_t)((1u << csz) - 1u);
   const uint32_t tmem_base = tmem_base_s;
   const uint32_t a_ring = tmem_base + (uint32_t)p.acc_cols;            // column offset of A stage 0
-  constexpr uint32_t kAStageCols = BF ? 32u : (uint32_t)NSPLIT * 32u;   // BF16: 16 cols hi | 16 cols lo
+  constexpr uint32_t kAStageCols = (uint32_t)NSPLIT * 32u;
 
   if (warp < 8) {
     const int q = warp & 3;                      // TMEM lane quarter == row quarter of the tile
@@ -598,11 +223,9 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
         const int src[8] = {i0.x, i0.y, i0.z, i0.w, i1.x, i1.y, i1.z, i1.w};
         mbar_wait(my_empty + 8 * sg, pg ^ 1u);             // slot released by the convert warp
         const uint32_t slot = my_slots + (uint32_t)sg * (uint32_t)kStageSlotBytes;
-        if (!TC_DBG(p, 2)) {
 #pragma unroll
-          for (int t = 0; t < 8; ++t)
-            cp_async16_row(slot + dst_off[t], base + (unsigned long long)(uint32_t)max(src[t], 0) * row_bytes, src[t]);
-        }
+        for (int t = 0; t < 8; ++t)
+          cp_async16_row(slot + dst_off[t], base + (unsigned long long)(uint32_t)max(src[t], 0) * row_bytes, src[t]);
         cp_async_mbar_arrive_noinc(my_full + 8 * sg);
         if (++sg == nsg) { sg = 0; pg ^= 1u; }
       }
@@ -617,52 +240,29 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
         mbar_wait(my_full + 8 * sg, pg);
         const uint32_t slot = my_slots + (uint32_t)sg * (uint32_t)kStageSlotBytes;
         float4 v[8];
-        if (!TC_DBG(p, 1)) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] = lds128(slot + src_off[j]);
-        } else {
-#pragma unroll
-          for (int j = 0; j < 8; ++j) v[j] = make_float4((float)it, 1.f, (float)lane, 2.f);
-        }
+        for (int j = 0; j < 8; ++j) v[j] = lds128(slot + src_off[j]);
         __syncwarp();
         if (lane == 0) mbar_arrive(my_empty + 8 * sg);     // release: the reads above are ordered before it
         if (++sg == nsg) { sg = 0; pg ^= 1u; }
         mbar_wait(a_empty + 8 * sa, pa ^ 1u);
         tc_fence_after();
         const uint32_t col = lane_base + a_ring + (uint32_t)sa * kAStageCols;
-        if constexpr (BF) {
-          // 32 K values of this row -> 16 packed bf16 words hi + 16 words lo (k even in the low half)
+#pragma unroll
+        for (int hh = 0; hh < 2; ++hh) {   // two 16-float halves keep the live registers down
           uint32_t hi[16], lo[16];
 #pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const float f[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
+          for (int j = 0; j < 4; ++j) {
+            const float4 fv = v[4 * hh + j];
+            const float f[4] = {fv.x, fv.y, fv.z, fv.w};
 #pragma unroll
-            for (int e = 0; e < 4; e += 2) {
-              const uint32_t h = cvt_bf16x2(f[e + 1], f[e]);
-              const float h0 = __uint_as_float(h << 16), h1 = __uint_as_float(h & 0xffff0000u);
-              hi[2 * j + e / 2] = h;
-              lo[2 * j + e / 2] = cvt_bf16x2(f[e + 1] - h1, f[e] - h0);
+            for (int e = 0; e < 4; ++e) {
+              hi[4 * j + e] = __float_as_uint(f[e]) & 0xffffe000u;
+              lo[4 * j + e] = __float_as_uint(f[e] - __uint_as_float(hi[4 * j + e]));
             }
           }
-          tc_st16(col, hi);
-          tc_st16(col + 16u, lo);
-        } else {
-#pragma unroll
-          for (int hh = 0; hh < 2; ++hh) {   // two 16-float halves keep the live registers down
-            uint32_t hi[16], lo[16];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float4 fv = v[4 * hh + j];
-              const float f[4] = {fv.x, fv.y, fv.z, fv.w};
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                hi[4 * j + e] = __float_as_uint(f[e]) & 0xffffe000u;
-                lo[4 * j + e] = __float_as_uint(f[e] - __uint_as_float(hi[4 * j + e]));
-              }
-            }
-            tc_st16(col + (uint32_t)(16 * hh), hi);
-            if (NSPLIT == 2) tc_st16(col + 32u + (uint32_t)(16 * hh), lo);
-          }
+          tc_st16(col + (uint32_t)(16 * hh), hi);
+          if (NSPLIT == 2) tc_st16(col + 32u + (uint32_t)(16 * hh), lo);
         }
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         tc_fence_before();
@@ -720,43 +320,34 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
     }
   } else if (warp == 8) {
     // =============================== MMA issuer ==========================================
-    const uint32_t idesc = BF ? umma_idesc_bf16(kTileM, c_out) : umma_idesc_tf32(kTileM, c_out);
-    const uint32_t idesc2 = BF ? umma_idesc_bf16(kTileM, 2 * c_out)   // merged [W_hi | W_lo] operand
-                               : umma_idesc_tf32(kTileM, 2 * c_out);
+    const uint32_t idesc = umma_idesc_tf32(kTileM, c_out);
+    const uint32_t idesc2 = umma_idesc_tf32(kTileM, 2 * c_out);   // merged [W_hi | W_lo] operand
     const int nmerge = p.nmerge;
     int sa = 0, sb = 0;
     uint32_t pa = 0, pb = 0;
     for (int it = 0; it < n_iters; ++it) {
       mbar_wait(a_full + 8 * sa, pa);
-      mbar_wait(b_full + 8 * sb, pb);   // BF16: already complete for the second K block of a stage
+      mbar_wait(b_full + 8 * sb, pb);
       tc_fence_after();
-      const bool last = it == n_iters - 1;
-      const bool b_done = !BF || (it & 1) || last;   // the weight stage is free after its last K block
       if (elect_one_sync()) {
         const uint32_t a_hi = a_ring + (uint32_t)sa * kAStageCols;   // lane 0, column offset
-        const uint32_t a_lo = a_hi + (BF ? 16u : 32u);
+        const uint32_t a_lo = a_hi + 32u;
         const uint32_t bstage = smem_base + (uint32_t)sb * (uint32_t)b_stage_bytes;
         const uint64_t b_hi = umma_desc_sw128(bstage);
         const uint64_t b_lo = umma_desc_sw128(bstage + b_part_bytes);
-        constexpr int KSTEPS = BF ? 2 : 4;           // 16 bf16 / 8 tf32 per MMA = 32 B of K either way
 #pragma unroll
-        for (int ks = 0; ks < (TC_DBG(p, 4) ? 0 : KSTEPS); ++ks) {
-          const uint64_t badv = (uint64_t)(ks * 2 + (BF ? (it & 1) * 4 : 0));
-          const uint32_t aadv = (uint32_t)(ks * 8);
+        for (int ks = 0; ks < 4; ++ks) {   // 8 tf32 per MMA = 32 B of K
+          const uint64_t badv = (uint64_t)(ks * 2);     // +32 B along K inside the 128-byte swizzled weight row
+          const uint32_t aadv = (uint32_t)(ks * 8);     // 8 TMEM columns per K step
           const uint32_t d = tmem_base;
           const uint32_t first = (it == 0 && ks == 0) ? 0u : 1u;
           if (nmerge) {
-            if constexpr (BF) {
-              tc_mma_bf16_ts(d, a_hi + aadv, b_hi + badv, idesc2, first);
-              tc_mma_bf16_ts(d, a_lo + aadv, b_hi + badv, idesc, 1u);
-            } else {
-              tc_mma_tf32_ts(d, a_hi + aadv, b_hi + badv, idesc2, first);
-              tc_mma_tf32_ts(d, a_lo + aadv, b_hi + badv, idesc, 1u);
-            }
-          } else if constexpr (BF) {
-            tc_mma_bf16_ts(d, a_lo + aadv, b_hi + badv, idesc, first);
-            tc_mma_bf16_ts(d, a_hi + aadv, b_lo + badv, idesc, 1u);
-            tc_mma_bf16_ts(d, a_hi + aadv, b_hi + badv, idesc, 1u);
+            // The hi and lo weight images are adjacent in the stage (same swizzle atoms), so one
+            // descriptor with N = 2*c_out multiplies A_hi by both: columns [0, c_out) collect
+            // hi*hi (+ lo*hi below), columns [c_out, 2 c_out) collect hi*lo.  2 MMAs, not 3; the
+            // epilogue adds the two column groups.
+            tc_mma_tf32_ts(d, a_hi + aadv, b_hi + badv, idesc2, first);
+            tc_mma_tf32_ts(d, a_lo + aadv, b_hi + badv, idesc, 1u);
           } else if (NSPLIT == 2) {
             tc_mma_tf32_ts(d, a_lo + aadv, b_hi + badv, idesc, first);
             tc_mma_tf32_ts(d, a_hi + aadv, b_lo + badv, idesc, 1u);
@@ -766,38 +357,30 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
           }
         }
         tc_commit(a_empty + 8 * sa);
-        if (b_done) {
-          if (csz > 1) tc_commit_mcast(b_empty + 8 * sb, cmask); else tc_commit(b_empty + 8 * sb);
-        }
-        if (last) tc_commit(accbar);
+        tc_commit(b_empty + 8 * sb);
+        if (it == n_iters - 1) tc_commit(accbar);
       }
       __syncwarp();
       if (++sa == nsa) { sa = 0; pa ^= 1u; }
-      if (b_done && ++sb == nsb) { sb = 0; pb ^= 1u; }
+      if (++sb == nsb) { sb = 0; pb ^= 1u; }
     }
   } else {
     // =============================== weight loader =======================================
     // Every CTA streams the whole weight tensor once per tile (515 tiles x 1.77 MB at C = 128): with the
-    // gather, the staging reads and the MMAs all disabled (BEVB200_TC_DBG=7) the kernel still takes
-    // 72 % of its time, i.e. the floor is the per-K-block synchronisation skeleton plus what every SM
-    // must ingest (weights: 16 KB per K block per CTA at C = 128, as much as the features).  Optional
-    // cluster mode: CTA rank r fetches slice r of a stage ONCE and multicasts it into the same ring slot
-    // of every CTA of the cluster (their b_full barriers count the bytes; a slot is rewritten only after
-    // the MMA warps of ALL cluster CTAs released it).  It halves the L2 reads but not the per-SM ingest
-    // and measured slower, so it is off by default.
+    // gather, the staging reads and the MMAs all disabled the kernel still took 72 % of its time (`dbg 7` of
+    // the since-removed timing-diagnostic build, profiles/r1_conv_v5_ablation.txt), i.e. the floor is the per-K-block synchronisation skeleton plus
+    // what every SM must ingest (weights: 16 KB per K block per CTA at C = 128, as much as the features).
+    // Multicasting the stages across a thread-block cluster halved the L2 reads but not the per-SM ingest
+    // and measured slower (DESIGN.md 4.6).
     if (lane == 0) {
-      const int n_bstages = BF ? (n_iters + 1) / 2 : n_iters;
-      const uint32_t crank = csz > 1 ? cluster_ctarank() : 0u;
-      const uint32_t slice = (uint32_t)b_stage_bytes / (uint32_t)csz;
-      const char *src = reinterpret_cast<const char *>(p.wpacked) + crank * slice;
+      const char *src = reinterpret_cast<const char *>(p.wpacked);
       int sb = 0;
       uint32_t pb = 1;   // an untouched stage counts as released
-      for (int it = 0; it < n_bstages; ++it) {
+      for (int it = 0; it < n_iters; ++it) {
         mbar_wait(b_empty + 8 * sb, pb);
         mbar_arrive_expect_tx(b_full + 8 * sb, (uint32_t)b_stage_bytes);
-        const uint32_t dst = smem_base + (uint32_t)sb * (uint32_t)b_stage_bytes + crank * slice;
-        if (csz > 1) bulk_copy_g2s_mcast(dst, src, slice, b_full + 8 * sb, cmask);
-        else bulk_copy_g2s(dst, src, slice, b_full + 8 * sb);
+        bulk_copy_g2s(smem_base + (uint32_t)sb * (uint32_t)b_stage_bytes, src, (uint32_t)b_stage_bytes,
+                      b_full + 8 * sb);
         src += b_stage_bytes;
         if (++sb == nsb) { sb = 0; pb ^= 1u; }
       }
@@ -806,7 +389,6 @@ __global__ void __launch_bounds__(kV4Threads, 2) spconv_tc_kernel_v5(const TcPar
   }
   tc_fence_before();
   __syncthreads();
-  if (csz > 1) cluster_sync_all();        // nobody leaves while a peer may still signal it
   if (warp == 8) {
     __syncwarp();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
@@ -842,36 +424,8 @@ int spconv_forward_simt(const float *features, const float *weight, const int32_
                         const float *shift, const float *residual, int relu, float *out,
                         cudaStream_t st);
 
-// BF16x3 weights: packed [nb64][hi | lo][Cout][64 bf16] in the swizzled smem image; K index
-// kk = kb64*64 + c (c in 0..63), 16-byte chunk (c / 8) XOR (n & 7), element (c % 8) inside the chunk.
-__global__ void spconv_pack_weights_bf16_kernel(const float *__restrict__ w, int kvol, int c_in, int c_in_eff,
-                                                int c_out, int nb64, uint16_t *__restrict__ packed) {
-  const long long total = (long long)nb64 * c_out * 64;
-  for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total;
-       t += (long long)gridDim.x * blockDim.x) {
-    const int c = (int)(t % 64);
-    const int n = (int)((t / 64) % c_out);
-    const int kb = (int)(t / (64ll * c_out));
-    const int kk = kb * 64 + c;
-    const int k = kk / c_in_eff, ci = kk % c_in_eff;
-    const float v = (k < kvol && ci < c_in) ? w[((long long)k * c_in + ci) * c_out + n] : 0.f;
-    uint32_t u = __float_as_uint(v);
-    u += 0x7fffu + ((u >> 16) & 1u);
-    const uint32_t hb = u >> 16;
-    const float lo = v - __uint_as_float(hb << 16);
-    uint32_t ul = __float_as_uint(lo);
-    ul += 0x7fffu + ((ul >> 16) & 1u);
-    const int pos = n * 64 + ((((c >> 3) ^ (n & 7)) << 3) | (c & 7));
-    packed[((long long)kb * 2 + 0) * c_out * 64 + pos] = (uint16_t)hb;
-    packed[((long long)kb * 2 + 1) * c_out * 64 + pos] = (uint16_t)(ul >> 16);
-  }
-}
-
-// kernel variant (BEVB200_SPCONV_TC_VARIANT): 6 (default for BF16X3: spconv_v6.cu -- pre-split operands
-// gathered straight into UMMA tiles, R row tiles per weight stage, persistent CTAs), 5 (A in tensor
-// memory, whole-line cp.async gather through swizzled staging slots + convert warps; the default for the
-// TF32 modes) or 4 (A in tensor memory, register gather + quad transposes).  4 and 5 are kept for A/B
-// measurements and are covered by tests/test_spconv_gpu.py.
+// Generation 6 (spconv_v6.cu: pre-split operands gathered straight into UMMA tiles, R row tiles per weight
+// stage, persistent CTAs) runs BF16X3; generation 5 (above) runs the TF32 modes.
 int spconv_v6_cin_eff(int c_in);
 bool spconv_v6_shape_ok(int c_in, int c_out, int kvol);
 size_t spconv_v6_packed_bytes(int c_in, int c_out, int kvol);
@@ -883,67 +437,47 @@ int spconv_v6_forward(const void *features_split, const void *packed, const int3
                       const float *scale, const float *shift, const float *residual, int relu, float *out,
                       void *out_split, cudaStream_t st);
 
-static int tc_variant(bool bf) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char *e = getenv("BEVB200_SPCONV_TC_VARIANT");
-    forced = e ? atoi(e) : 0;
-  }
-  if (forced == 4 || forced == 5) return forced;
-  return bf ? 6 : 5;
-}
 static bool use_v6(int c_in, int c_out, int kvol, int precision) {
-  return precision == BEVB200_PREC_BF16X3 && tc_variant(true) == 6 && spconv_v6_shape_ok(c_in, c_out, kvol);
+  return precision == BEVB200_PREC_BF16X3 && spconv_v6_shape_ok(c_in, c_out, kvol);
 }
 // for spconv_bwd.cu: does this (shape, precision) run on generation 6, i.e. on split row images?
 bool spconv_tc_runs_on_split_images(int c_in, int c_out, int kvol, int precision) {
   return use_v6(c_in, c_out, kvol, precision);
 }
 
-// Input channels the kernel runs with: narrow inputs (conv_input: Cin = 5) are zero-padded to 8
-// (v5; 16 for the older variants), other counts to the next power of two up to 128.  0 = no
-// tensor-core form.
-static int tc_cin_eff(int c_in, int precision) {
-  const int lo = tc_variant(precision == BEVB200_PREC_BF16X3) == 5 ? 8 : 16;
-  for (int e = lo; e <= 128; e <<= 1)
+// Input channels the TF32 kernel runs with: narrow inputs (conv_input: Cin = 5) are zero-padded to 8,
+// other counts to the next power of two up to 128.  0 = no tensor-core form.
+static int tc_cin_eff(int c_in) {
+  for (int e = 8; e <= 128; e <<= 1)
     if (c_in <= e) return e;
   return 0;
 }
 
-static bool tc_shape_ok(int c_in, int c_out, int kvol, int precision) {
-  return (c_out == 16 || c_out == 32 || c_out == 64 || c_out == 128) && c_in >= 1 &&
-         tc_cin_eff(c_in, precision) != 0 && kvol >= 1 && kvol <= 27;
+static bool tc_shape_ok(int c_in, int c_out, int kvol) {
+  return (c_out == 16 || c_out == 32 || c_out == 64 || c_out == 128) && c_in >= 1 && tc_cin_eff(c_in) != 0 &&
+         kvol >= 1 && kvol <= 27;
 }
 
 int spconv_padded_channels(int c_in, int precision) {
   if (precision == BEVB200_PREC_FP32 || c_in < 1) return c_in;
-  if (precision == BEVB200_PREC_BF16X3 && tc_variant(true) == 6) return c_in;   // the split pass pads
-  const int e = tc_cin_eff(c_in, precision);
+  if (precision == BEVB200_PREC_BF16X3) return c_in;   // the split pass pads
+  const int e = tc_cin_eff(c_in);
   return e ? e : c_in;
 }
 
 static int tc_nkb(int c_in_eff, int kvol) { return (kvol * c_in_eff + kKBlock - 1) / kKBlock; }
 
 size_t spconv_packed_bytes(int c_in, int c_out, int kvol, int precision) {
-  if (use_v6(c_in, c_out, kvol, precision)) return spconv_v6_packed_bytes(c_in, c_out, kvol);
-  if (!tc_shape_ok(c_in, c_out, kvol, precision)) return 0;
-  const int ce = tc_cin_eff(c_in, precision);
-  if (precision == BEVB200_PREC_BF16X3)
-    return (size_t)((tc_nkb(ce, kvol) + 1) / 2) * 2 * c_out * 64 * sizeof(uint16_t);
+  if (precision == BEVB200_PREC_BF16X3) return spconv_v6_packed_bytes(c_in, c_out, kvol);
+  if (!tc_shape_ok(c_in, c_out, kvol)) return 0;
   const int nsplit = precision == BEVB200_PREC_TF32X3 ? 2 : 1;
-  return (size_t)tc_nkb(ce, kvol) * nsplit * c_out * 32 * sizeof(float);
+  return (size_t)tc_nkb(tc_cin_eff(c_in), kvol) * nsplit * c_out * 32 * sizeof(float);
 }
 
 int spconv_pack_weights(const float *weight, int c_in, int c_out, int kvol, int precision,
                         float *packed, cudaStream_t st) {
-  if (use_v6(c_in, c_out, kvol, precision)) return spconv_v6_pack_weights(weight, c_in, c_out, kvol, packed, st);
-  const int ce = tc_cin_eff(c_in, precision);
-  if (precision == BEVB200_PREC_BF16X3) {
-    const int nb64 = (tc_nkb(ce, kvol) + 1) / 2;
-    BEVB200_LAUNCH(spconv_pack_weights_bf16_kernel, grid_for((long long)nb64 * c_out * 64, 256), 256, 0, st,
-                   weight, kvol, c_in, ce, c_out, nb64, (uint16_t *)packed);
-    return BEVB200_OK;
-  }
+  if (precision == BEVB200_PREC_BF16X3) return spconv_v6_pack_weights(weight, c_in, c_out, kvol, packed, st);
+  const int ce = tc_cin_eff(c_in);
   const int nsplit = precision == BEVB200_PREC_TF32X3 ? 2 : 1;
   const int nkb = tc_nkb(ce, kvol);
   BEVB200_LAUNCH(spconv_pack_weights_kernel, grid_for((long long)nkb * c_out * 32, 256), 256, 0, st,
@@ -1000,12 +534,13 @@ int spconv_forward_tc(const float *features, const float *weight, const float *p
     if (wtmp) cudaFreeAsync(wtmp, st);
     return rc;
   }
+  // BF16X3 shapes generation 6 cannot take (unaligned out / residual) and shapes / alignments the UMMA path
+  // cannot take: exact-fp32 SIMT kernel
   const int c_in_real = c_in;
-  const int c_eff = tc_shape_ok(c_in, c_out, kvol, precision) ? tc_cin_eff(c_in, precision) : 0;
+  const int c_eff = precision != BEVB200_PREC_BF16X3 && tc_shape_ok(c_in, c_out, kvol) ? tc_cin_eff(c_in) : 0;
   const bool ok = c_eff != 0 && (c_eff != c_in || (uintptr_t)features % 16 == 0) &&
                   ((uintptr_t)out % 16 == 0) && (residual == nullptr || (uintptr_t)residual % 16 == 0);
   if (!ok) {
-    // shapes / alignments the UMMA path cannot take: exact-fp32 SIMT kernel
     if (weight == nullptr) {
       snprintf(g_last_error, sizeof(g_last_error), "spconv_forward: shape needs the unpacked weights");
       return BEVB200_EINVAL;
@@ -1013,8 +548,6 @@ int spconv_forward_tc(const float *features, const float *weight, const float *p
     return spconv_forward_simt(features, weight, nbr, n_in, n_out, c_in, c_out, kvol, scale, shift,
                                residual, relu, out, st);
   }
-  const bool bf = precision == BEVB200_PREC_BF16X3;
-  const int variant = tc_variant(bf) == 4 ? 4 : 5;
   // stream-ordered temporaries, released on every exit path
   struct Temps {
     cudaStream_t st;
@@ -1034,13 +567,9 @@ int spconv_forward_tc(const float *features, const float *weight, const float *p
     features = padded;
     c_in = c_eff;
   }
-  const int nsplit = precision == BEVB200_PREC_TF32X3 ? 2 : 1;   // tf32 parts (unused in BF16 mode)
-  const int nkb = tc_nkb(c_in, kvol);
+  const int nsplit = precision == BEVB200_PREC_TF32X3 ? 2 : 1;   // tf32 parts
   int cin_shift = 0;
   while ((1 << cin_shift) < c_in) ++cin_shift;
-  const int acc_cols = c_out < 32 ? 32 : c_out;
-  const int nbr_bytes = kvol * kTileM * 4;
-  const int grid_tiles = (n_out + kTileM - 1) / kTileM;
 
   float *&packed = tmp.packed;
   const float *wpacked = packed_in;
@@ -1051,120 +580,36 @@ int spconv_forward_tc(const float *features, const float *weight, const float *p
     wpacked = packed;
   }
 
-  {
-    TcParamsV4 p4;
-    p4.features = features; p4.nbr = nbr; p4.scale = scale; p4.shift = shift; p4.residual = residual;
-    p4.out = out; p4.n_in = n_in; p4.n_out = n_out; p4.c_in = c_in; p4.c_out = c_out; p4.kvol = kvol;
-    p4.relu = relu; p4.nkb = nkb; p4.cin_shift = cin_shift; p4.wpacked = wpacked;
-    static int merge_env = -1;
-    if (merge_env < 0) {
-      const char *e = getenv("BEVB200_SPCONV_NMERGE");
-      merge_env = e ? atoi(e) : 1;
-    }
-    p4.dbg = 0;
-#ifdef BEVB200_TC_PROFILE
-    {
-      static int dbg_env = -1;
-      if (dbg_env < 0) {
-        const char *e = getenv("BEVB200_TC_DBG");
-        dbg_env = e ? atoi(e) : 0;
-      }
-      p4.dbg = dbg_env;
-    }
-#endif
-    p4.nmerge = (merge_env && (nsplit == 2 || bf) && c_out <= 64) ? 1 : 0;
-    p4.acc_cols = p4.nmerge ? (2 * c_out < 32 ? 32 : 2 * c_out) : acc_cols;
-    {
-      // dev profiling: BEVB200_TC_PROF=<device pointer of 8 int64 counters, hex>
-      static long long *prof_ptr = (long long *)-1;
-      if (prof_ptr == (long long *)-1) {
-        const char *e = getenv("BEVB200_TC_PROF");
-        prof_ptr = e ? (long long *)strtoull(e, nullptr, 16) : nullptr;
-      }
-      p4.prof = prof_ptr;
-    }
-    // 256 TMEM columns per CTA (two CTAs per SM): accumulator + A ring (>= 2 stages)
-    const int a_stage_cols = bf ? 32 : nsplit * 32;
-    p4.nsa = (256 - p4.acc_cols) / a_stage_cols;
-    if (p4.nsa > 4) p4.nsa = 4;
-    p4.tmem_cols = 256;
-    const int b_stage4 = (bf ? 2 : nsplit) * c_out * 128;
-    int nsb4;
-    size_t smem4;
-    if (variant == 5) {
-      // per CTA (two per SM): 1 KB alignment slack + weight ring + neighbour table + 4 quarters x nsg
-      // staging slots of 4 KB.  As many slots as fit beside a 2-stage weight ring, then the ring
-      // takes what is left.
-      const int budget = 111 * 1024;
-      p4.nbr_bytes = ((kvol + 1) * kTileM * 4 + 127) / 128 * 128;   // + one all -1 row (K tail padding)
-      const int avail = budget - 1024 - p4.nbr_bytes;
-      int nsg = (avail - 2 * b_stage4) / (4 * kStageSlotBytes);
-      if (nsg > kMaxGatherSlots) nsg = kMaxGatherSlots;
-      {
-        static int nsg_env = -1;
-        if (nsg_env < 0) {
-          const char *e = getenv("BEVB200_TC_NSG");
-          nsg_env = e ? atoi(e) : 0;
-        }
-        if (nsg_env >= 2 && nsg_env < nsg) nsg = nsg_env;
-      }
-      BEVB200_REQUIRE(nsg >= 2, "shared memory budget: no room for two gather slots");
-      p4.nsg = nsg;
-      nsb4 = (avail - nsg * 4 * kStageSlotBytes) / b_stage4;
-      if (nsb4 > kMaxStages) nsb4 = kMaxStages;
-      smem4 = (size_t)nsb4 * b_stage4 + p4.nbr_bytes + (size_t)nsg * 4 * kStageSlotBytes + 1024;
-    } else {
-      p4.nsg = 0;
-      p4.nbr_bytes = nbr_bytes;
-      nsb4 = (110 * 1024 - nbr_bytes - 1024) / b_stage4;
-      if (nsb4 > kMaxStages) nsb4 = kMaxStages;
-      if (nsb4 < 2) nsb4 = 2;
-      smem4 = (size_t)nsb4 * b_stage4 + nbr_bytes + 1024;
-    }
-    p4.nsb = nsb4;
-    // v5: thread-block clusters can multicast the weight stages (BEVB200_SPCONV_CLUSTER=2|4).  Measured:
-    // no gain (2.54 / 2.69 ms vs 2.41 ms for the 20 convs) -- the floor is what each SM has to ingest
-    // (16 KB of weights + 16 KB of features per K block per CTA at C = 128), not the L2 read rate, so
-    // the default stays 1.
-    static int csz_env = -1;
-    if (csz_env < 0) {
-      const char *e = getenv("BEVB200_SPCONV_CLUSTER");
-      csz_env = e ? atoi(e) : 0;
-    }
-    int csz = 1;
-    if (variant == 5) {
-      csz = csz_env ? csz_env : 1;
-      if (csz != 1 && csz != 2 && csz != 4) csz = 1;
-    }
-    p4.csz = csz;
-    const int grid4 = (grid_tiles + csz - 1) / csz * csz;
-    auto launch = [&](auto kernel) -> int {
-      BEVB200_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem4));
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3(grid4);
-      cfg.blockDim = dim3(kV4Threads);
-      cfg.dynamicSmemBytes = smem4;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = csz;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      BEVB200_CUDA(cudaLaunchKernelEx(&cfg, kernel, p4));
-      return BEVB200_OK;
-    };
-    int lrc;
-    if (variant == 5)
-      lrc = bf ? launch(spconv_tc_kernel_v5<3>)
-               : (nsplit == 2 ? launch(spconv_tc_kernel_v5<2>) : launch(spconv_tc_kernel_v5<1>));
-    else
-      lrc = bf ? launch(spconv_tc_kernel_v4<3>)
-               : (nsplit == 2 ? launch(spconv_tc_kernel_v4<2>) : launch(spconv_tc_kernel_v4<1>));
-    if (lrc) return lrc;
-    ++g_launch_count;
+  TcParams p;
+  p.features = features; p.nbr = nbr; p.scale = scale; p.shift = shift; p.residual = residual;
+  p.out = out; p.n_in = n_in; p.n_out = n_out; p.c_in = c_in; p.c_out = c_out; p.kvol = kvol;
+  p.relu = relu; p.nkb = tc_nkb(c_in, kvol); p.cin_shift = cin_shift; p.wpacked = wpacked;
+  p.nmerge = (nsplit == 2 && c_out <= 64) ? 1 : 0;
+  p.acc_cols = p.nmerge ? (2 * c_out < 32 ? 32 : 2 * c_out) : (c_out < 32 ? 32 : c_out);
+  // 256 TMEM columns per CTA (two CTAs per SM): accumulator + A ring (>= 2 stages)
+  p.nsa = (256 - p.acc_cols) / (nsplit * 32);
+  if (p.nsa > 4) p.nsa = 4;
+  p.tmem_cols = 256;
+  // per CTA (two per SM): 1 KB alignment slack + weight ring + neighbour table + 4 quarters x nsg
+  // staging slots of 4 KB.  As many slots as fit beside a 2-stage weight ring, then the ring
+  // takes what is left.
+  const int b_stage = nsplit * c_out * 128;
+  const int budget = 111 * 1024;
+  p.nbr_bytes = ((kvol + 1) * kTileM * 4 + 127) / 128 * 128;   // + one all -1 row (K tail padding)
+  const int avail = budget - 1024 - p.nbr_bytes;
+  p.nsg = (avail - 2 * b_stage) / (4 * kStageSlotBytes);
+  if (p.nsg > kMaxGatherSlots) p.nsg = kMaxGatherSlots;
+  BEVB200_REQUIRE(p.nsg >= 2, "shared memory budget: no room for two gather slots");
+  p.nsb = (avail - p.nsg * 4 * kStageSlotBytes) / b_stage;
+  if (p.nsb > kMaxStages) p.nsb = kMaxStages;
+  const size_t smem = (size_t)p.nsb * b_stage + p.nbr_bytes + (size_t)p.nsg * 4 * kStageSlotBytes + 1024;
+  const int grid = (n_out + kTileM - 1) / kTileM;
+  if (nsplit == 2) {
+    BEVB200_CUDA(cudaFuncSetAttribute(spconv_tc_kernel_v5<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    BEVB200_LAUNCH(spconv_tc_kernel_v5<2>, grid, kTcThreads, smem, st, p);
+  } else {
+    BEVB200_CUDA(cudaFuncSetAttribute(spconv_tc_kernel_v5<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    BEVB200_LAUNCH(spconv_tc_kernel_v5<1>, grid, kTcThreads, smem, st, p);
   }
   return BEVB200_OK;
 }

@@ -27,22 +27,15 @@
 // Warp roles (10 warps): 0-7 gather (row quarter = warp & 3; the two halves take alternate items) and
 // epilogue (TMEM lane quarter = warp & 3, the halves split the columns); 8 MMA issuer (one elected
 // lane) + TMEM allocation; 9 weight stream (cp.async.bulk ring).
-//   * TMA ROW GATHER (kTma, BEVB200_V6_TMA=1, c_in >= 32; measured and NOT the default).  Warp 10 stages
-//     the operand tiles with cp.async.bulk.tensor ... tile::gather4: one instruction copies the 128-byte
-//     K block of FOUR rows (indices straight from the neighbour table, -1 / out-of-range rows arrive as
-//     zeros) into the SWIZZLE_128B tile and completes on the stage's mbarrier by byte count; warps 0-7
-//     only run epilogues.  The copies bypass the LSU data pipe, but the TMA unit's gather4 rate is the
-//     new bound and it is lower: see the note at the launch.
-#include <cuda.h>
-#include <stdlib.h>
-
+// A TMA row gather (cp.async.bulk.tensor ... tile::gather4, four rows per instruction, from an eleventh warp)
+// was measured 2x slower than the cp.async gather and removed: the TMA unit's gather4 rate is lower than what
+// the LDGSTS gather sustains; measurement in profiles/r2_gather4_probe.txt.
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
 namespace bevb200 {
 
-constexpr int kV6Threads = 10 * 32;      // LDGSTS gather (c_in = 16)
-constexpr int kV6ThreadsTma = 11 * 32;   // + the TMA gather warp
+constexpr int kV6Threads = 10 * 32;
 constexpr int kV6TileM = 128;
 constexpr int kV6AStageBytes = kV6TileM * 128;   // 128 rows x 128 B
 constexpr int kV6MaxA = 12, kV6MaxB = 4;
@@ -66,9 +59,6 @@ struct V6Params {
   int merged;                   // 1: A_hi x [W_hi | W_lo] (Cout <= 64); 0: three products (Cout = 128)
   int nsa, nsb, b_stage_bytes;
   int tmem_cols;
-  int proxy_fence;               // tuning: fence.proxy.async before the MMAs of an item (BEVB200_V6_FENCE)
-  int lag;                       // tuning: signal an item this many of the warp's items later (BEVB200_V6_LAG: 0 / 1 / 2)
-  int gfence;                    // tuning: fence.proxy.async in the gather warps before the arrive (BEVB200_V6_GFENCE)
 };
 
 __device__ __forceinline__ void tc_mma_bf16_ss(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc,
@@ -169,18 +159,7 @@ __device__ __forceinline__ void v6_store_chunk(const V6Params &p, float (&acc)[N
   }
 }
 
-// 4 rows x 128 B of the split image -> 512 contiguous bytes of a SWIZZLE_128B tile (tools/gather4_probe.cu)
-__device__ __forceinline__ void tma_gather4(uint32_t dst_smem, const CUtensorMap *map, int col, int r0, int r1,
-                                            int r2, int r3, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes "
-      "[%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
-      ::"r"(dst_smem), "l"(map), "r"(col), "r"(r0), "r"(r1), "r"(r2), "r"(r3), "r"(bar) : "memory");
-}
-
-template <bool kTma>
-__global__ void __launch_bounds__(kTma ? kV6ThreadsTma : kV6Threads, 2)
-spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
+__global__ void __launch_bounds__(kV6Threads, 2) spconv_v6_kernel(const V6Params p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   __shared__ uint64_t bars[2 * kV6MaxA + 2 * kV6MaxB + 2];
@@ -197,7 +176,7 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
 
   if (tid == 0) {
     for (int s = 0; s < nsa; ++s) {
-      mbar_init(a_full + 8 * s, kTma ? 1 : 4);   // the producer's expect_tx / one arrival per gather warp of the stage
+      mbar_init(a_full + 8 * s, 4);   // one arrival per gather warp of the stage
       mbar_init(a_empty + 8 * s, 1);
     }
     for (int s = 0; s < nsb; ++s) {
@@ -219,8 +198,7 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
   const uint32_t tmem_base = tmem_base_s;
 
   // Programmatic dependent launch: everything above (barriers, TMEM) ran while the previous kernel of the stream was
-  // still draining; its results (feature image, row count) are only touched below.  Without the launch attribute both
-  // instructions are no-ops.
+  // still draining; its results (feature image, row count) are only touched below.
   asm volatile("griddepcontrol.wait;" ::: "memory");
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
@@ -230,7 +208,6 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
   const int n_tiles = (n_out + kV6TileM - 1) / kV6TileM;
   const int t_begin = (int)((long long)n_tiles * blockIdx.x / gridDim.x);
   const int t_end = (int)((long long)n_tiles * (blockIdx.x + 1) / gridDim.x);
-  const int r_max = 1 << p.r_shift;
 
   if (warp < 8) {
     // =============================== gather + epilogue ===================================
@@ -249,17 +226,15 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
     uint32_t dst_off[8];
 #pragma unroll
     for (int t = 0; t < 8; ++t) dst_off[t] = (uint32_t)((q * 32 + 8 * m + t) * 128 + (c << 4));
-    // an item is signalled `lag` of this warp's items later (see the hand-off below): that needs spare stages
-    const int lag = (p.lag >= 2 && nsa >= 6) ? 2 : ((p.lag >= 1 && nsa >= 3) ? 1 : 0);
-    const bool gfence = p.gfence != 0;
-    int pend = -1, pend0 = -1;   // stages whose copies are committed but not yet signalled (newest, older)
+    // an item is signalled one of this warp's items later (see the hand-off below): that needs a spare stage
+    const bool lag = nsa >= 3;
+    int pend = -1;          // stage whose copies are committed but not yet signalled
     int gs = 0;             // A ring stage / phase of the first item of the current group
     uint32_t gph = 0, acc_ph = 0;
     for (int tb = t_begin; tb < t_end;) {
       int rs = p.r_shift;
       while ((1 << rs) > t_end - tb) --rs;
       const int r_cur = 1 << rs, n_items = nkb << rs;
-      if constexpr (!kTma) {
       int s = gs + par;     // ... of this warp's first item of the group (nsa >= 2)
       uint32_t ph = gph;
       if (s >= nsa) { s -= nsa; ph ^= 1u; }
@@ -323,26 +298,17 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
         // kernel.  Instead the warp commits the item as a cp.async group and signals the PREVIOUS item with ONE
         // arrive once that group has landed (wait_group 1): by then its copies have had a whole item's time.
         asm volatile("cp.async.commit_group;" ::: "memory");
-        if (lag == 2) {
-          if (pend0 >= 0) {
-            asm volatile("cp.async.wait_group 2;" ::: "memory");
-            if (gfence) fence_proxy_async();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(a_full + 8 * pend0);
-          }
-          pend0 = pend;
-          pend = s;
-        } else if (lag == 1) {
+        if (lag) {
           if (pend >= 0) {
             asm volatile("cp.async.wait_group 1;" ::: "memory");
-            if (gfence) fence_proxy_async();
+            fence_proxy_async();
             __syncwarp();
             if (lane == 0) mbar_arrive(a_full + 8 * pend);
           }
           pend = s;
         } else {
           asm volatile("cp.async.wait_group 0;" ::: "memory");
-          if (gfence) fence_proxy_async();
+          fence_proxy_async();
           __syncwarp();
           if (lane == 0) mbar_arrive(a_full + 8 * s);
         }
@@ -350,17 +316,13 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
         if (s >= nsa) { s -= nsa; ph ^= 1u; }
         }
       }
-      if (pend0 >= 0 || pend >= 0) {        // the last item(s) of the group
+      if (pend >= 0) {                      // the last item of the group
         asm volatile("cp.async.wait_group 0;" ::: "memory");
-        if (gfence) fence_proxy_async();
+        fence_proxy_async();
         __syncwarp();
-        if (lane == 0) {
-          if (pend0 >= 0) mbar_arrive(a_full + 8 * pend0);
-          if (pend >= 0) mbar_arrive(a_full + 8 * pend);
-        }
-        pend0 = pend = -1;
+        if (lane == 0) mbar_arrive(a_full + 8 * pend);
+        pend = -1;
       }
-      }  // !kTma
       // ------------------------------- epilogue of the group --------------------------------
       mbar_wait(acc_full, acc_ph);
       acc_ph ^= 1u;
@@ -425,7 +387,6 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
         const bool b_done = r == r_cur - 1 && (!merged || (kb & 1) || kb == nkb - 1);
         if (b_new) mbar_wait(b_full + 8 * sb, pb);
         mbar_wait(a_full + 8 * sa, pa);
-        if (p.proxy_fence) fence_proxy_async();
         tc_fence_after();
         if (elect_one_sync()) {
           const uint32_t a_base = a_ring + (uint32_t)sa * (uint32_t)kV6AStageBytes;
@@ -480,60 +441,7 @@ spconv_v6_kernel(const V6Params p, const __grid_constant__ CUtensorMap amap) {
       }
     }
     __syncwarp();
-  } else if constexpr (kTma) {
-    // =============================== TMA row gather (warp 10) ============================
-    // Lane l owns rows 4 l .. 4 l + 3 of every tile: one gather4 per lane and item, 512 bytes each.
-    const int cin_shift = p.cin_shift, cin_mask = p.c_in - 1, kvol = p.kvol;
-    const long long nbr_stride = p.nbr_stride;
-    const bool vec = (nbr_stride & 3) == 0 && (reinterpret_cast<uintptr_t>(p.nbr) & 15) == 0;
-    int s = 0;
-    uint32_t ph = 0;
-    for (int tb = t_begin; tb < t_end;) {
-      int rs = p.r_shift;
-      while ((1 << rs) > t_end - tb) --rs;
-      const int r_cur = 1 << rs, n_items = nkb << rs;
-      auto load_idx = [&](int i) {
-        const int kb = i >> rs, r = i & (r_cur - 1);
-        const int row = (tb + r) * kV6TileM + 4 * lane;
-        const int k0 = (kb * 32) >> cin_shift;
-        int4 v = make_int4(-1, -1, -1, -1);
-        if (k0 < kvol) {
-          const int32_t *src = p.nbr + (long long)k0 * nbr_stride + row;
-          if (vec && row + 3 < n_out) {
-            v = __ldg(reinterpret_cast<const int4 *>(src));
-          } else {
-            if (row < n_out) v.x = __ldg(src);
-            if (row + 1 < n_out) v.y = __ldg(src + 1);
-            if (row + 2 < n_out) v.z = __ldg(src + 2);
-            if (row + 3 < n_out) v.w = __ldg(src + 3);
-          }
-        }
-        return v;
-      };
-      constexpr int PF = 4;      // items whose indices are in flight ahead of the copies
-      int4 vq[PF];
-#pragma unroll
-      for (int j = 0; j < PF; ++j) vq[j] = j < n_items ? load_idx(j) : make_int4(-1, -1, -1, -1);
-      for (int ibase = 0; ibase < n_items; ibase += PF) {
-#pragma unroll
-        for (int j = 0; j < PF; ++j) {
-          const int i = ibase + j;
-          if (i >= n_items) break;
-          const int4 v = vq[j];
-          if (i + PF < n_items) vq[j] = load_idx(i + PF);
-          const int col = (((i >> rs) * 32) & cin_mask) * 2;     // bf16 elements into the row image
-          mbar_wait(a_empty + 8 * s, ph ^ 1u);
-          if (lane == 0) mbar_arrive_expect_tx(a_full + 8 * s, (uint32_t)kV6AStageBytes);
-          __syncwarp();
-          tma_gather4(a_ring + (uint32_t)s * (uint32_t)kV6AStageBytes + (uint32_t)lane * 512u, &amap, col, v.x, v.y,
-                      v.z, v.w, a_full + 8 * s);
-          if (++s == nsa) { s = 0; ph ^= 1u; }
-        }
-      }
-      tb += r_cur;
-    }
   }
-  (void)r_max;
   tc_fence_before();
   __syncthreads();
   if (warp == 8) {
@@ -662,34 +570,6 @@ int spconv_v6_split_rows(const float *features, int n_cap, const int32_t *n_dev,
   return BEVB200_OK;
 }
 
-// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda)
-typedef CUresult (*V6EncodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static V6EncodeTiled v6_encode_fn() {
-  static V6EncodeTiled fn = [] {
-    void *f = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      f = nullptr;
-    return (V6EncodeTiled)f;
-  }();
-  return fn;
-}
-// the split image as a 2-D bf16 tensor [rows][c_in * 2], one 128-byte K block of one row per box
-static bool v6_row_map(const void *split, int rows, int c_in, CUtensorMap *map) {
-  V6EncodeTiled enc = v6_encode_fn();
-  if (!enc) return false;
-  const cuuint64_t dims[2] = {(cuuint64_t)c_in * 2, (cuuint64_t)(rows > 0 ? rows : 1)};
-  const cuuint64_t strides[1] = {(cuuint64_t)c_in * 4};
-  const cuuint32_t box[2] = {64, 1};
-  const cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(split), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 // split image with an explicit padded channel count (multiple of 16, >= c_in): the filter-gradient kernel wants
 // whole 128-byte slabs (spconv_wgrad_tc.cu)
 int spconv_v6_split_rows_padded(const float *features, int n, int c_in, int c_eff, void *split, cudaStream_t st) {
@@ -698,11 +578,6 @@ int spconv_v6_split_rows_padded(const float *features, int n, int c_in, int c_ef
   BEVB200_LAUNCH(spconv_v6_split_rows_kernel, grid_for((long long)n * (c_eff / 8), 256), 256, 0, st, features, n,
                  (const int32_t *)nullptr, c_in, c_eff, (uint8_t *)split);
   return BEVB200_OK;
-}
-
-static int env_int(const char *name, int dflt) {
-  const char *e = getenv(name);
-  return e ? atoi(e) : dflt;
 }
 
 // features_split: split image with c_in (multiple of 16, <= 128) channels per row.
@@ -748,71 +623,39 @@ int spconv_v6_forward_ex(const void *features_split, const void *packed, const i
   while ((1 << p.cin_shift) < c_in) ++p.cin_shift;
   p.merged = c_out <= 64 ? 1 : 0;
   p.acc_cols = p.merged ? (2 * c_out < 32 ? 32 : 2 * c_out) : c_out;
-  // tuning: BEVB200_V6_CTAS=1 runs ONE persistent CTA per SM (all 512 TMEM columns, ~225 KB of shared memory:
-  // more A stages in flight per SM because only one weight ring is resident) instead of two
-  static const int ctas_env = env_int("BEVB200_V6_CTAS", 2);
-  const int ctas = ctas_env == 1 ? 1 : 2;
-  p.tmem_cols = ctas == 1 ? 512 : 256;
-  static const int fence_env = env_int("BEVB200_V6_FENCE", 0);
-  p.proxy_fence = fence_env;
-  static const int lag_env = env_int("BEVB200_V6_LAG", 1);
-  p.lag = lag_env;
-  static const int gfence_env = env_int("BEVB200_V6_GFENCE", 1);
-  p.gfence = gfence_env;
+  // two persistent CTAs per SM, each with half of the 512 TMEM columns and of the shared memory
+  p.tmem_cols = 256;
   int r = p.tmem_cols / p.acc_cols;
   if (r > 4) r = 4;
-  static const int r_env = env_int("BEVB200_V6_R", 0);
-  if (r_env >= 1 && r_env < r) r = r_env;
   p.r_shift = 0;
   while ((2 << p.r_shift) <= r) ++p.r_shift;
   p.b_stage_bytes = p.merged ? 2 * c_out * 128 : c_out * 128;
-  // per CTA (two per SM): 1 KB alignment slack + weight ring + A ring
-  const int budget = (ctas == 1 ? 225 : 111) * 1024 - 1024;
-  static const int nsb_env = env_int("BEVB200_V6_NSB", 0);
-  p.nsb = nsb_env >= 2 && nsb_env <= kV6MaxB ? nsb_env : ((!p.merged || p.b_stage_bytes <= 8192) ? 3 : 2);
+  // per CTA: 1 KB alignment slack + weight ring + A ring
+  const int budget = 111 * 1024 - 1024;
+  p.nsb = (!p.merged || p.b_stage_bytes <= 8192) ? 3 : 2;
   p.nsa = (budget - p.nsb * p.b_stage_bytes) / kV6AStageBytes;
   if (p.nsa > kV6MaxA) p.nsa = kV6MaxA;
-  static const int nsa_env = env_int("BEVB200_V6_NSA", 0);
-  if (nsa_env >= 2 && nsa_env < p.nsa) p.nsa = nsa_env;
   BEVB200_REQUIRE(p.nsa >= 2, "shared memory budget: no room for two A stages");
   const size_t smem = (size_t)p.nsb * p.b_stage_bytes + (size_t)p.nsa * kV6AStageBytes + 1024;
   const int n_tiles = (n_out + kV6TileM - 1) / kV6TileM;
-  int grid = ctas * kNumSMs;
+  int grid = 2 * kNumSMs;
   if (grid > n_tiles) grid = n_tiles;
-  // operand gather: LDGSTS.  BEVB200_V6_TMA=1 selects the TMA gather4 producer for c_in >= 32 -- bit-identical
-  // results, but measured 2x SLOWER (5.10 vs 2.74 ms for the 21 convs): one warp issues a gather4 every ~90-190 clk
-  // and the unit tops out at ~23 B/clk/SM on valid rows, ~13 B/clk/SM with 55 % out-of-range rows, against the
-  // ~26 B/clk/SM the LDGSTS kernel sustains end to end (tools/gather4_probe.cu, profiles/r2_gather4_probe.txt).
-  static const int tma_env = env_int("BEVB200_V6_TMA", 0);
-  CUtensorMap amap;
-  memset(&amap, 0, sizeof(amap));
-  if (tma_env != 0 && c_in >= 32) {
-    BEVB200_REQUIRE(v6_row_map(features_split, n_in, c_in, &amap), "cuTensorMapEncodeTiled failed for the row image");
-    BEVB200_CUDA(cudaFuncSetAttribute(spconv_v6_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    BEVB200_LAUNCH(spconv_v6_kernel<true>, grid, kV6ThreadsTma, smem, st, p, amap);
-  } else {
-    BEVB200_CUDA(cudaFuncSetAttribute(spconv_v6_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // BEVB200_V6_PDL=1 (default): programmatic stream serialisation -- the kernel's prologue overlaps the tail of
-    // the previous kernel in the stream (21 back-to-back convs per frame)
-    static const int pdl_env = env_int("BEVB200_V6_PDL", 1);
-    if (pdl_env) {
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3((unsigned)grid);
-      cfg.blockDim = dim3((unsigned)kV6Threads);
-      cfg.dynamicSmemBytes = smem;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[0].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      BEVB200_CUDA(cudaLaunchKernelEx(&cfg, spconv_v6_kernel<false>, p, amap));
-      ++g_launch_count;
-    } else {
-      BEVB200_LAUNCH(spconv_v6_kernel<false>, grid, kV6Threads, smem, st, p, amap);
-    }
-  }
+  BEVB200_CUDA(cudaFuncSetAttribute(spconv_v6_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // programmatic stream serialisation: the kernel's prologue overlaps the tail of the previous kernel in the
+  // stream (21 back-to-back convs per frame)
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3((unsigned)grid);
+  cfg.blockDim = dim3((unsigned)kV6Threads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  BEVB200_CUDA(cudaLaunchKernelEx(&cfg, spconv_v6_kernel, p));
+  ++g_launch_count;
   return BEVB200_OK;
 }
 

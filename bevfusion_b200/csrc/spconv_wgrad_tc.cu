@@ -46,7 +46,6 @@ struct WgtParams {
   int m_blocks;                // accumulator row blocks (two feature slabs each): s_a / 2
   int stages, stage_bytes;
   int tmem_cols;
-  int ablate;                  // dev: 1 = no MMAs (hand-offs only), 2 = no feature-row copies (BEVB200_WGRAD_ABLATE)
 };
 
 // UMMA shared-memory descriptor, MN-major, SWIZZLE_128B (cute/atom/mma_traits_sm100.hpp, canonical layout
@@ -193,14 +192,12 @@ spconv_wgrad_tc_kernel(const WgtParams p, const __grid_constant__ CUtensorMap gm
         load_idx(t + 2, idx1);
         mbar_wait(empty + 8 * s, ph ^ 1u);
         const uint32_t a_stage = ring + (uint32_t)s * stage_bytes;
-        if (!(p.ablate & 2)) {
 #pragma unroll
-          for (int j = 0; j < kWgtMaxUnits; ++j) {
-            if (j < n_units) {
-              const uint32_t dst = a_stage + u_dst[j];
-              const unsigned long long src = fbase + (unsigned long long)(uint32_t)max(cur[j], 0) * row_bytes + u_src[j];
-              for (int i = 0; i < n_a; ++i) cp_async16_row(dst + (uint32_t)i * kSlab, src + (unsigned)(i * 128), cur[j]);
-            }
+        for (int j = 0; j < kWgtMaxUnits; ++j) {
+          if (j < n_units) {
+            const uint32_t dst = a_stage + u_dst[j];
+            const unsigned long long src = fbase + (unsigned long long)(uint32_t)max(cur[j], 0) * row_bytes + u_src[j];
+            for (int i = 0; i < n_a; ++i) cp_async16_row(dst + (uint32_t)i * kSlab, src + (unsigned)(i * 128), cur[j]);
           }
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
@@ -288,14 +285,12 @@ spconv_wgrad_tc_kernel(const WgtParams p, const __grid_constant__ CUtensorMap gm
         if (elect_one_sync()) {
           const uint32_t a_stage = ring + (uint32_t)s * stage_bytes;
           const uint32_t b_stage = a_stage + (uint32_t)s_a * kSlab;
-          if (!(p.ablate & 1)) {
 #pragma unroll
-            for (int ks = 0; ks < R / 16; ++ks) {
-              const uint64_t bdesc = umma_desc_mn_sw128(b_stage + (uint32_t)(ks * 2048), kSlab);
-              for (int mb = 0; mb < p.m_blocks; ++mb) {
-                const uint64_t adesc = umma_desc_mn_sw128(a_stage + (uint32_t)(2 * mb) * kSlab + (uint32_t)(ks * 2048), kSlab);
-                wgt_mma(tmem_base + (uint32_t)(mb * n2), adesc, bdesc, idesc, (t == t_begin && ks == 0) ? 0u : 1u);
-              }
+          for (int ks = 0; ks < R / 16; ++ks) {
+            const uint64_t bdesc = umma_desc_mn_sw128(b_stage + (uint32_t)(ks * 2048), kSlab);
+            for (int mb = 0; mb < p.m_blocks; ++mb) {
+              const uint64_t adesc = umma_desc_mn_sw128(a_stage + (uint32_t)(2 * mb) * kSlab + (uint32_t)(ks * 2048), kSlab);
+              wgt_mma(tmem_base + (uint32_t)(mb * n2), adesc, bdesc, idesc, (t == t_begin && ks == 0) ? 0u : 1u);
             }
           }
           tc_commit(empty + 8 * s);
@@ -395,8 +390,6 @@ static WgtPlan wgt_plan(int n_out, int c_in, int c_out, int kvol) {
   if (g > kvol) g = kvol;
   if (w.n_a == 1 && g > 4) g = 4;                    // measured: 4 offsets per item beat 8 / 16 for 32-channel slabs
   if (w.n_a == 1 && (g & 1)) ++g;                    // 32-channel slabs pair up two offsets per block
-  static const int g_env = [] { const char *e = getenv("BEVB200_WGRAD_G"); return e ? atoi(e) : 0; }();
-  if (g_env >= 1 && g_env < g) g = (w.n_a == 1 && (g_env & 1)) ? g_env + 1 : g_env;
   w.g = g;
   w.n_kgroups = (kvol + g - 1) / g;
   w.s_a = g * w.n_a;
@@ -404,9 +397,7 @@ static WgtPlan wgt_plan(int n_out, int c_in, int c_out, int kvol) {
   w.tmem_cols = 32;
   while (w.tmem_cols < w.m_blocks * n2) w.tmem_cols <<= 1;
   // rows per stage: 16 / 32 / 64 / 128, a stage of at most 64 KB and at most 8 copy units per gather lane
-  static const int r_env = [] { const char *e = getenv("BEVB200_WGRAD_ROWS"); return e ? atoi(e) : 0; }();
   int rows = 128;
-  if (r_env == 16 || r_env == 32 || r_env == 64 || r_env == 128) rows = r_env;
   while (rows > 16 && ((w.s_a + w.n_b) * rows * 128 > 64 * 1024 || g * (rows / 4) > 8 * kWgtMaxUnits)) rows >>= 1;
   w.rows = rows;
   w.stage_bytes = (w.s_a + w.n_b) * rows * 128;
@@ -459,8 +450,6 @@ int spconv_wgrad_tc(const float *features, const float *out_grad, const int32_t 
   p.stage_bytes = w.stage_bytes; p.stages = w.stages;
   p.tmem_cols = w.tmem_cols;
   BEVB200_REQUIRE(p.tmem_cols <= 512 && p.stages >= 2, "filter gradient tile does not fit");
-  static const int ablate_env = [] { const char *e = getenv("BEVB200_WGRAD_ABLATE"); return e ? atoi(e) : 0; }();
-  p.ablate = ablate_env;
   // out-grad split image as a 2-D bf16 tensor [n_out][co_eff * 2]; one box = `rows` rows x 128 B
   WgtEncodeTiled enc = wgt_encode_fn();
   BEVB200_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available");

@@ -21,11 +21,7 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "WAIT_LOOP:\n\t"
-#ifdef BEVB200_TC_NOHINT
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-#else
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, 0x989680;\n\t"   // suspend, do not spin
-#endif
       "@p bra WAIT_DONE;\n\t"
       "bra WAIT_LOOP;\n\t"
       "WAIT_DONE:\n\t}"
@@ -48,26 +44,6 @@ __device__ __forceinline__ bool elect_one_sync() {
       "selp.b32 %0, 1, 0, P;\n\t}"
       : "=r"(pred));
   return pred != 0;
-}
-__device__ __forceinline__ void bulk_copy_g2s_mcast(uint32_t dst_smem, const void *src, uint32_t bytes,
-                                                    uint32_t bar, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster "
-      "[%0], [%1], %2, [%3], %4;"
-      ::"r"(dst_smem), "l"(src), "r"(bytes), "r"(bar), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ void tc_commit_mcast(uint32_t bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(bar), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
 }
 __device__ __forceinline__ void fence_proxy_async() {
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");

@@ -42,6 +42,18 @@ def test_product_does_not_import_oracle():
         assert not re.search(r"^\s*(from|import)\s+oracle\b", src, re.M), path
 
 
+def test_library_reads_only_documented_switches():
+    """The native library reads one environment variable, BEVB200_WGRAD_TC (documented in the header), and its
+    build defines no preprocessor switches: every kernel path a user can reach is a path the tests cover."""
+    import glob, os, re
+    from bevfusion_b200 import build
+    names = set()
+    for path in glob.glob(os.path.join(build.CSRC, "*")):
+        names |= set(re.findall(r'"(BEVB200_\w*)"', open(path).read()))
+    assert names == {"BEVB200_WGRAD_TC"}
+    assert not any(f.startswith("-D") for f in build.FLAGS), build.FLAGS
+
+
 def test_conv_output_size_matches_reference_formula():
     from bevfusion_b200.spconv import ops
     import oracle
